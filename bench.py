@@ -2,6 +2,7 @@
 """bench.py -- CenterTrack per-frame inference hot path on B200 (contract: see DESIGN.md section 6).
 
   python bench.py --gpus N --steps K --warmup W [--batch B] [--config CFG] [--precision P] [--impl reference]
+                   [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (default = BASELINE.json configs[1]): DLA-34 coco_tracking, 512x512, bf16, synthetic frame pairs, K=100.
@@ -171,15 +172,10 @@ def run_reference(args, rank, world):
   for _ in range(min(args.warmup, 1)):
     _oracle_step(args.config, 1)
   t, thr = 0.0, 1
-  steps = min(args.steps, 6)
-  done = 0
+  steps = args.steps
   for _ in range(steps):
     dt, thr, _n = _oracle_step(args.config, frames_per_step)
     t += dt
-    done += 1
-    if t > 60.0:                                        # bounded sample on any host
-      break
-  steps = done
   fps = steps * frames_per_step / t
   line = {'impl': 'reference', 'metric': metric_name(args.config), 'value': fps, 'unit': 'frames/s', 'n_gpus': args.gpus,
           'steps': steps, 'warmup': min(args.warmup, 1), 'ms_per_step': 1000 * t / steps,
@@ -416,6 +412,23 @@ def stock_pytorch_leg(sd, heads, B, H, W, dev, wt, steps=3, warmup=2):
   return res
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, runner):
+  """What a caller of StreamRunner.step_device holds after the last timed step, as DIR/<name>.npy: the packed decode
+  records [B,K,F] and, with device tracking, the track table [B,T,CT_TRK_FLOATS] and the per-stream counts [B,2]."""
+  arrays = {'records': runner.rec.cpu().numpy()}
+  if runner.tracker is not None:
+    arrays['tracks'] = runner.tracker.tracks.cpu().numpy()
+    arrays['track_counts'] = runner.tracker.counts.cpu().numpy().astype(np.float64)
+  total = sum(a.nbytes for a in arrays.values())
+  assert total <= DUMP_LIMIT_BYTES, 'output dump of %d bytes exceeds %d' % (total, DUMP_LIMIT_BYTES)
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in arrays.items():
+    np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def main():
   ap = argparse.ArgumentParser()
   ap.add_argument('--gpus', type=int, default=1)
@@ -432,7 +445,12 @@ def main():
   ap.add_argument('--no-accurate', action='store_true', help='skip the bf16x3 (<= 1e-3) engine leg of the default run')
   ap.add_argument('--host-tracking', action='store_true',
                   help='round-1 mode: pre_hm supplied by the host, no association on the device')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='write the records and track tables of the last timed step to DIR/<name>.npy (inputs are seeded: '
+                       'the same arguments give the same inputs, so two builds can be compared output for output)')
   args = ap.parse_args()
+  if args.dump_outputs and args.impl != 'b200':
+    ap.error('--dump-outputs dumps the device path (--impl b200)')
   # stdout carries exactly ONE JSON line: everything any library writes to fd 1 during the run (NCCL prints a version
   # banner there) is sent to stderr, and the result line goes to the saved descriptor (see _emit)
   global _REAL_STDOUT
@@ -510,6 +528,8 @@ def main():
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
   clocks = sampler.summary() if rank == 0 else None
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, runner)
   ms_per_step = ms / args.steps
   value = world * B * args.steps / (ms / 1000.0)
 

@@ -6,8 +6,11 @@
 Inputs and weights are pure functions of seeds (oracle/weights.py, numpy RandomState) so the GPU box
 regenerates them bit-identically without the reference; only the reference's OUTPUTS are stored.
 """
+import hashlib
+import json
 import os
 import sys
+import time
 
 import numpy as np
 import torch
@@ -423,8 +426,36 @@ def gen_host():
   print('host_pre', len(data), 'arrays')
 
 
+DIGESTS = 'reference_digests.json'
+
+
+def golden_digest(path):
+  """sha256 of a fixture's content: the parsed JSON, or every array's name, dtype, shape and bytes of an .npz."""
+  h = hashlib.sha256()
+  if path.endswith('.json'):
+    h.update(json.dumps(json.load(open(path)), sort_keys=True).encode())
+    return h.hexdigest()
+  with np.load(path) as z:
+    for k in sorted(z.files):
+      a = np.ascontiguousarray(z[k])
+      h.update(('%s|%s|%s|' % (k, a.dtype.str, a.shape)).encode())
+      h.update(a.tobytes())
+  return h.hexdigest()
+
+
+def write_digests(names):
+  """Record what the reference produced in DIGESTS, so that the committed fixtures can be checked against this run
+  where the reference is not at hand (tests/test_golden_fresh.py)."""
+  path = os.path.join(OUT, DIGESTS)
+  d = json.load(open(path)) if os.path.exists(path) else {}
+  d.update({n: golden_digest(os.path.join(OUT, n)) for n in names})
+  with open(path, 'w') as f:
+    json.dump(d, f, indent=1, sort_keys=True)
+
+
 if __name__ == '__main__':
   os.makedirs(OUT, exist_ok=True)
+  t0 = time.time()
   torch.manual_seed(0)
   which = sys.argv[1:] or ['net', 'generic', 'e2e', 'decode', 'post', 'track', 'host', 'opts', 'flip']
   rh.install()
@@ -447,3 +478,4 @@ if __name__ == '__main__':
     gen_dataset_info()
   if 'flip' in which:
     gen_flip()
+  write_digests(sorted(n for n in os.listdir(OUT) if n != DIGESTS and os.path.getmtime(os.path.join(OUT, n)) >= t0))

@@ -1,26 +1,38 @@
-"""Golden freshness: when the reference checkout is present (the build container), re-run oracle/gen_golden.py on
-the UNMODIFIED reference into a scratch directory and require the committed tests/golden fixtures to be what the
-reference produces today (same keys, integers exact, floats to 1e-5 -- CPU conv summation order may change with
-the thread count).  Skipped on the GPU box (no /root/reference there)."""
+"""Golden freshness: the committed tests/golden fixtures must be what the UNMODIFIED reference produces.
+
+Every run of oracle/gen_golden.py on the reference records a sha256 of each fixture it wrote in
+tests/golden/reference_digests.json; the committed fixtures must hash to exactly that (no checkout needed).  When
+CT_REF_ROOT names a CenterTrack checkout, the generator is also re-run on it into a scratch directory and its output
+compared with the committed fixtures (same keys, integers exact, floats to 1e-5 -- CPU conv summation order may change
+with the thread count)."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
-import pytest
+
+from gen_golden import DIGESTS, golden_digest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get('CT_REF_ROOT', '/root/reference')
+REF = os.environ.get('CT_REF_ROOT', '')
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'src', 'lib')), reason='reference checkout not present')
+SHIM_RECORD = 'shim_reference_run.npz'       # made by tests/shim_driver.py from the reference's scripts
+
+
 def test_committed_goldens_are_what_the_reference_produces(tmp_path, golden_dir):
+  want = json.load(open(os.path.join(golden_dir, DIGESTS)))
+  assert sorted(want) == sorted(set(os.listdir(golden_dir)) - {DIGESTS, SHIM_RECORD})
+  for name in sorted(want):
+    assert golden_digest(os.path.join(golden_dir, name)) == want[name], name + ' is not what the reference produced'
+  if not (REF and os.path.isdir(os.path.join(REF, 'src', 'lib'))):
+    return
   env = dict(os.environ, CT_GOLDEN_OUT=str(tmp_path))
   r = subprocess.run([sys.executable, os.path.join(ROOT, 'oracle', 'gen_golden.py'), 'net', 'generic', 'decode', 'post', 'track', 'host',
                       'opts', 'e2e', 'flip'], capture_output=True, text=True, timeout=1500, env=env)
   assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-  fresh = sorted(os.listdir(str(tmp_path)))
+  fresh = sorted(set(os.listdir(str(tmp_path))) - {DIGESTS})
   assert fresh, 'generator wrote nothing'
   for name in fresh:
     a_path, b_path = os.path.join(str(tmp_path), name), os.path.join(golden_dir, name)
