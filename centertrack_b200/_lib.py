@@ -66,7 +66,11 @@ class TrackDesc(C.Structure):
       ('max_age', C.c_int32), ('inp_h', C.c_int32), ('inp_w', C.c_int32),
       ('records', C.c_void_p), ('trans_out_inv', C.c_void_p), ('trans_input', C.c_void_p),
       ('tracks', C.c_void_p), ('counts', C.c_void_p), ('boxes', C.c_void_p),
+      ('assign', C.c_int32), ('public_det', C.c_void_p), ('public_count', C.c_void_p), ('max_public', C.c_int32),
   ]
+
+
+CT_ASSIGN_GREEDY, CT_ASSIGN_HUNGARIAN = 0, 1
 
 
 EXPORTS = ['ct_packed_weight_bytes', 'ct_pack_weights', 'ct_conv_forward', 'ct_stem_forward',

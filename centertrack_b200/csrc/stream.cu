@@ -7,6 +7,8 @@
 //   ct_warp_affine_normalize   Detector.pre_process's cv2.warpAffine(INTER_LINEAR) + (x/255 - mean)/std + HWC->CHW
 //                    (detector.py:207-226), cv2's fixed-point bilinear restated
 // All HBM-bound byte/index work: one pass over the data, coalesced, no tensor cores.
+#include <math_constants.h>
+
 #include "common.cuh"
 
 namespace ctb {
@@ -65,6 +67,175 @@ __device__ double gaussian_radius_f64(double h, double w) {
   return fmin(r1, fmin(r2, r3));
 }
 
+// dynamic shared memory of the greedy step (track table, detections, per-row bookkeeping) ...
+__host__ __device__ inline size_t track_smem_greedy(int K, int T) {
+  return ((size_t)T * TF + (size_t)K * TF + 3 * (size_t)K + T) * 4 + (2 * (size_t)K + 2 * (size_t)T) * 4 + 64;
+}
+// ... and the scratch of the assignment solver and the public-detection births behind it (8-byte aligned):
+// doubles spc[T], v[T], u[K]; ints path[T], row4col[T], remaining[T], col_seen[T], col4row[K], row_seen[K],
+// rejected[K], claimed[K], born[K].  Rows of the solver are the shorter side (<= K), columns the longer (<= T).
+__host__ __device__ inline size_t track_smem_scratch_offset(int K, int T) {
+  return (track_smem_greedy(K, T) + 7) & ~(size_t)7;
+}
+__host__ __device__ inline size_t track_smem_full(int K, int T) {
+  return track_smem_scratch_offset(K, T) + (size_t)T * (2 * 8 + 4 * 4) + (size_t)K * (8 + 5 * 4);
+}
+
+// Gated association cost of (detection i, track j) as tracker.py::_gated_cost + hungarian_assignment build it:
+// float64 of the float32 squared distance between the detection's predicted previous centre and the track centre,
+// or exactly 1e18 when the pair is blocked (distance above either box area, or different classes).
+struct GatedCost {
+  const float* old; const float* det; const float* px; const float* py; const float* isz; const float* tsz;
+  __device__ __forceinline__ double operator()(int i, int j) const {
+    const float* t = old + (size_t)j * TF;
+    const float dx = __fsub_rn(t[CT_TRK_CT], px[i]), dy = __fsub_rn(t[CT_TRK_CT + 1], py[i]);
+    const float dist = __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
+    const bool blocked = dist > tsz[j] || dist > isz[i] || t[CT_TRK_CLASS] != det[(size_t)i * TF + CT_TRK_CLASS];
+    return blocked ? 1e18 : (double)dist;
+  }
+};
+
+// One candidate column of a Dijkstra round: reduced cost, position in `remaining`, column still unassigned.
+struct LsapPick { double v; int pos; bool free; };
+
+// scipy's tie rule (rectangular_lsap.cpp): the minimum reduced cost; among equal minima the LAST unassigned column in
+// scan order if there is one, else the FIRST.  Commutative and associative over disjoint sets of positions, so it
+// runs as a butterfly.
+__device__ __forceinline__ LsapPick lsap_better(LsapPick a, LsapPick b) {
+  if (b.pos < 0) return a;
+  if (a.pos < 0) return b;
+  if (b.v < a.v) return b;
+  if (a.v < b.v) return a;
+  if (a.free || b.free) {
+    if (a.free && b.free) return b.pos > a.pos ? b : a;
+    return a.free ? a : b;
+  }
+  return b.pos < a.pos ? b : a;
+}
+
+// Minimum-cost assignment of the N x M gated cost matrix by ONE warp, pair for pair what scipy's
+// linear_sum_assignment returns: Crouse's shortest augmenting path (scipy/optimize/rectangular_lsap.cpp), restated
+// in Python in tests/lsap_restated.py.  N > M solves the transpose (rows = tracks).  Each round the lanes relax their
+// columns of `remaining` and pick the next column by warp shuffles, in the same float64 operation order as scipy.
+// Results: s_match[det] = track of a kept pair (cost <= 1e16), s_rej[det] = track of a pair forced through a blocked
+// cell, s_taken[track] = 1 for every paired track.
+__device__ void lsap_warp(const GatedCost& cost, int N, int M, int lane, double* spc, double* v, double* u, int* path,
+                          int* row4col, int* remaining, int* col_seen, int* col4row, int* row_seen, int* s_match,
+                          int* s_rej, int* s_taken) {
+  const unsigned full = 0xffffffffu;
+  const bool tr = N > M;
+  const int nr = tr ? M : N, nc = tr ? N : M;
+  for (int c = lane; c < nc; c += 32) { v[c] = 0.0; row4col[c] = -1; }
+  for (int r = lane; r < nr; r += 32) { u[r] = 0.0; col4row[r] = -1; }
+  for (int i = lane; i < N; i += 32) s_rej[i] = -1;
+  __syncwarp();
+  for (int cur = 0; cur < nr; ++cur) {
+    for (int c = lane; c < nc; c += 32) { remaining[c] = nc - 1 - c; spc[c] = CUDART_INF; col_seen[c] = 0; }
+    for (int r = lane; r < nr; r += 32) row_seen[r] = 0;
+    __syncwarp();
+    double minVal = 0.0;
+    int i = cur, sink = -1, nrem = nc;
+    while (sink < 0) {
+      if (lane == 0) row_seen[i] = 1;
+      const double ui = u[i];
+      LsapPick best = {CUDART_INF, -1, false};
+      for (int it = lane; it < nrem; it += 32) {
+        const int j = remaining[it];
+        const double r = __dsub_rn(__dsub_rn(__dadd_rn(minVal, tr ? cost(j, i) : cost(i, j)), ui), v[j]);
+        double s = spc[j];
+        if (r < s) { path[j] = i; spc[j] = r; s = r; }
+        const LsapPick p = {s, it, row4col[j] == -1};
+        best = lsap_better(best, p);
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        LsapPick p;
+        p.v = __shfl_xor_sync(full, best.v, o);
+        p.pos = __shfl_xor_sync(full, best.pos, o);
+        p.free = __shfl_xor_sync(full, (int)best.free, o) != 0;
+        best = lsap_better(best, p);
+      }
+      minVal = best.v;
+      const int j = remaining[best.pos];
+      const int owner = row4col[j];
+      __syncwarp();                                   // every lane is done with remaining / spc of this round
+      if (lane == 0) { col_seen[j] = 1; remaining[best.pos] = remaining[nrem - 1]; }
+      --nrem;
+      if (owner == -1) sink = j; else i = owner;
+      __syncwarp();
+    }
+    // dual update (u of the rows and v of the columns reached this augmentation), then flip the path
+    for (int r = lane; r < nr; r += 32)
+      if (row_seen[r] && r != cur) u[r] = __dadd_rn(u[r], __dsub_rn(minVal, spc[col4row[r]]));
+    if (lane == 0) u[cur] = __dadd_rn(u[cur], minVal);
+    for (int c = lane; c < nc; c += 32)
+      if (col_seen[c]) v[c] = __dsub_rn(v[c], __dsub_rn(minVal, spc[c]));
+    __syncwarp();
+    if (lane == 0) {
+      int j = sink;
+      while (true) {
+        const int r = path[j];
+        row4col[j] = r;
+        const int nxt = col4row[r];
+        col4row[r] = j;
+        j = nxt;
+        if (r == cur) break;
+      }
+    }
+    __syncwarp();
+  }
+  for (int r = lane; r < nr; r += 32) {
+    const int c = col4row[r];
+    const int det = tr ? c : r, trk = tr ? r : c;
+    s_taken[trk] = 1;
+    if (cost(det, trk) <= 1e16) s_match[det] = trk; else s_rej[det] = trk;
+  }
+}
+
+// MOT public-detection births (tracker.py:83-103, host: tracker.py::_public_births) by one warp: each public
+// detection in order claims the first nearest (float32 squared distance of the predicted previous centre) detection
+// not yet matched or claimed, if that distance is below the detection's box area; a claimed detection confident enough
+// to start a track is appended to born[].  Returns the number of births.  Runs only if some detection is unmatched.
+__device__ int public_births_warp(const float* pub, int P, int N, int lane, const float* px, const float* py,
+                                  const float* isz, const float* det, float new_thresh, const int* s_match,
+                                  int* claimed, int* born) {
+  const unsigned full = 0xffffffffu;
+  bool any_free = false;
+  for (int i = lane; i < N; i += 32) {
+    claimed[i] = s_match[i] >= 0;
+    any_free |= s_match[i] < 0;
+  }
+  __syncwarp();
+  if (!__any_sync(full, any_free)) return 0;
+  int nb = 0;
+  for (int p = 0; p < P; ++p) {
+    const float qx = pub[2 * p], qy = pub[2 * p + 1];
+    float best = 3.0e38f;
+    int bi = 0x7fffffff;
+    for (int i = lane; i < N; i += 32) {
+      const float dx = __fsub_rn(px[i], qx), dy = __fsub_rn(py[i], qy);
+      const float c = claimed[i] ? 1e18f : __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
+      if (c < best) { best = c; bi = i; }              // ascending i per lane: first minimum kept
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ov = __shfl_xor_sync(full, best, o);
+      const int oi = __shfl_xor_sync(full, bi, o);
+      if (ov < best || (ov == best && oi < bi)) { best = ov; bi = oi; }
+    }
+    __syncwarp();
+    if (bi < N && best < isz[bi]) {
+      if (lane == 0) claimed[bi] = 1;
+      if (det[(size_t)bi * TF + CT_TRK_SCORE] > new_thresh) {
+        if (lane == 0) born[nb] = bi;
+        ++nb;
+      }
+    }
+    __syncwarp();
+  }
+  return nb;
+}
+
 __global__ void __launch_bounds__(TRK_THREADS)
 track_step_kernel(const TrackArgs a) {
   extern __shared__ __align__(16) unsigned char tsm[];
@@ -81,9 +252,23 @@ track_step_kernel(const TrackArgs a) {
   int* s_taken = s_match + K;                                   // [T]
   int* s_pos_det = s_taken + T;                                 // [K] output slot of det or -1
   int* s_pos_trk = s_pos_det + K;                               // [T] output slot of a coasting track or -1
+  // solver / public-birth scratch: only present (and only touched) with --hungarian or public detections
+  double* s_spc = reinterpret_cast<double*>(tsm + track_smem_scratch_offset(K, T));   // [T]
+  double* s_v = s_spc + T;                                      // [T]
+  double* s_u = s_v + T;                                        // [K]
+  int* s_path = reinterpret_cast<int*>(s_u + K);                // [T]
+  int* s_row4col = s_path + T;                                  // [T]
+  int* s_remaining = s_row4col + T;                             // [T]
+  int* s_col_seen = s_remaining + T;                            // [T]
+  int* s_col4row = s_col_seen + T;                              // [K]
+  int* s_row_seen = s_col4row + K;                              // [K]
+  int* s_rej = s_row_seen + K;                                  // [K] track of a rejected (forced) pair or -1
+  int* s_claimed = s_rej + K;                                   // [K]
+  int* s_born = s_claimed + K;                                  // [K] public births in claim order
+  const bool hung = d.assign == CT_ASSIGN_HUNGARIAN;
   __shared__ float red_v[TRK_THREADS / 32];
   __shared__ int red_j[TRK_THREADS / 32];
-  __shared__ int s_n, s_total, s_ids;
+  __shared__ int s_n, s_total, s_ids, s_nborn;
 
   int M = d.counts[b * 2 + 0];
   if (M > T) M = T;
@@ -132,10 +317,19 @@ track_step_kernel(const TrackArgs a) {
   }
   __syncthreads();
 
+  if (hung) {
+    // ---- --hungarian (tracker.py:52-72): minimum-cost assignment by warp 0
+    if (warp == 0) {
+      const GatedCost cost = {s_old, s_det, s_px, s_py, s_isz, s_tsz};
+      lsap_warp(cost, N, M, lane, s_spc, s_v, s_u, s_path, s_row4col, s_remaining, s_col_seen, s_col4row, s_row_seen,
+                s_match, s_rej, s_taken);
+    }
+    __syncthreads();
+  }
   // ---- greedy assignment (tracker.py:129-138): detections in score order take their nearest free, valid track;
   //      argmin ties -> lowest track index
   const float INF = 3.0e38f;
-  for (int i = 0; i < N && M > 0; ++i) {
+  for (int i = 0; i < N && M > 0 && !hung; ++i) {
     const float px = s_px[i], py = s_py[i], isz = s_isz[i], icls = s_det[(size_t)i * TF + CT_TRK_CLASS];
     float best = INF;
     int bj = 0x7fffffff;
@@ -164,7 +358,20 @@ track_step_kernel(const TrackArgs a) {
     __syncthreads();
   }
 
-  // ---- output order (tracker.py:74-127): matched detections, then new tracks, then coasting tracks
+  // ---- MOT public detections (tracker.py:83-103): births only on detections a public detection claims
+  if (d.public_det) {
+    if (warp == 0) {
+      int P = min(d.public_count[b], d.max_public);
+      P = P > 0 ? P : 0;
+      const int nb = public_births_warp(d.public_det + (size_t)b * d.max_public * 2, P, N, lane, s_px, s_py, s_isz,
+                                        s_det, d.new_thresh, s_match, s_claimed, s_born);
+      if (lane == 0) s_nborn = nb;
+    }
+    __syncthreads();
+  }
+
+  // ---- output order (tracker.py:74-127): matched detections, then new tracks, then coasting tracks; with
+  //      --hungarian the detections / tracks of rejected pairs follow the naturally unmatched ones, in pair order
   if (tid == 0) {
     int pos = 0, ids = id_count;
     for (int i = 0; i < N; ++i) {
@@ -176,18 +383,46 @@ track_step_kernel(const TrackArgs a) {
         if (pos < T) s_pos_det[i] = pos++;
       }
     }
-    for (int i = 0; i < N; ++i) {
-      if (s_match[i] >= 0) continue;
-      float* o = s_det + (size_t)i * TF;
-      if (o[CT_TRK_SCORE] > d.new_thresh) {
+    if (d.public_det) {
+      for (int k = 0; k < s_nborn; ++k) {
+        const int i = s_born[k];
+        float* o = s_det + (size_t)i * TF;
         ++ids;
         o[CT_TRK_ID] = (float)ids; o[CT_TRK_AGE] = 1.f; o[CT_TRK_ACTIVE] = 1.f;
         if (pos < T) s_pos_det[i] = pos++;
+      }
+    } else {
+      for (int i = 0; i < N; ++i) {
+        if (s_match[i] >= 0 || (hung && s_rej[i] >= 0)) continue;
+        float* o = s_det + (size_t)i * TF;
+        if (o[CT_TRK_SCORE] > d.new_thresh) {
+          ++ids;
+          o[CT_TRK_ID] = (float)ids; o[CT_TRK_AGE] = 1.f; o[CT_TRK_ACTIVE] = 1.f;
+          if (pos < T) s_pos_det[i] = pos++;
+        }
+      }
+      for (int i = 0; i < N && hung; ++i) {
+        if (s_rej[i] < 0) continue;
+        float* o = s_det + (size_t)i * TF;
+        if (o[CT_TRK_SCORE] > d.new_thresh) {
+          ++ids;
+          o[CT_TRK_ID] = (float)ids; o[CT_TRK_AGE] = 1.f; o[CT_TRK_ACTIVE] = 1.f;
+          if (pos < T) s_pos_det[i] = pos++;
+        }
       }
     }
     for (int j = 0; j < M; ++j) {
       s_pos_trk[j] = -1;
       if (s_taken[j]) continue;
+      float* t = s_old + (size_t)j * TF;
+      if (t[CT_TRK_AGE] < (float)d.max_age) {
+        t[CT_TRK_AGE] += 1.f; t[CT_TRK_ACTIVE] = 0.f;
+        if (pos < T) s_pos_trk[j] = pos++;
+      }
+    }
+    for (int i = 0; i < N && hung; ++i) {
+      const int j = s_rej[i];
+      if (j < 0) continue;
       float* t = s_old + (size_t)j * TF;
       if (t[CT_TRK_AGE] < (float)d.max_age) {
         t[CT_TRK_AGE] += 1.f; t[CT_TRK_ACTIVE] = 0.f;
@@ -333,8 +568,7 @@ extern "C" int ct_flip_merge(const float* in2, float* out, int32_t C, int32_t H,
 }
 
 extern "C" int64_t ct_track_smem_bytes(int32_t K, int32_t max_tracks) {
-  return (int64_t)((size_t)max_tracks * TF + (size_t)K * TF + 3 * (size_t)K + max_tracks) * 4 +
-         (int64_t)(2 * (size_t)K + 2 * (size_t)max_tracks) * 4 + 64;
+  return (int64_t)track_smem_full(K, max_tracks);
 }
 
 extern "C" int ct_track_step(const ct_track_desc* d, void* stream) {
@@ -342,7 +576,12 @@ extern "C" int ct_track_step(const ct_track_desc* d, void* stream) {
   CT_REQUIRE(d->B > 0 && d->K > 0 && d->F >= CT_REC_HEADS && d->max_tracks >= d->K, "bad shape");
   CT_REQUIRE(d->rec_tracking < 0 || d->rec_tracking + 2 <= d->F, "tracking offset outside the record");
   CT_REQUIRE(d->boxes == nullptr || (d->trans_input != nullptr && d->inp_h > 0 && d->inp_w > 0), "boxes need trans_input");
-  const size_t smem = (size_t)ct_track_smem_bytes(d->K, d->max_tracks);
+  CT_REQUIRE(d->assign == CT_ASSIGN_GREEDY || d->assign == CT_ASSIGN_HUNGARIAN, "unknown assign mode");
+  CT_REQUIRE(d->public_det == nullptr || d->public_count != nullptr, "public_det needs public_count");
+  CT_REQUIRE(d->max_public >= 0, "max_public < 0");
+  // greedy with private births launches exactly as it did before the solver existed: no scratch
+  const bool scratch = d->assign != CT_ASSIGN_GREEDY || d->public_det != nullptr;
+  const size_t smem = scratch ? track_smem_full(d->K, d->max_tracks) : track_smem_greedy(d->K, d->max_tracks);
   CT_REQUIRE(smem <= 200 * 1024, "track table does not fit in shared memory (lower max_tracks)");
   if (smem > 48 * 1024)
     CT_CUDA_OK(cudaFuncSetAttribute(track_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

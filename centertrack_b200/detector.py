@@ -47,6 +47,28 @@ class _StageClock(object):
     return out
 
 
+def trans_bbox(bbox, trans, width, height):
+  """Box corners through a 2x3 affine map, clipped to [0, width-1] x [0, height-1] (detector.py:242-251)."""
+  corners = np.asarray(bbox, dtype=np.float32).reshape(2, 2)
+  moved = np.stack([affine_transform(corners[0], trans), affine_transform(corners[1], trans)]).astype(np.float32)
+  return np.clip(moved, 0, np.array([width - 1, height - 1], dtype=np.float32)).reshape(4)
+
+
+def prior_splats(dets, trans_input, inp_w, inp_h, pre_thresh):
+  """The tracks the prior heat-map is drawn from (detector.py:259-276): active, score >= pre_thresh and a box of
+  positive size once mapped onto the network input.  Yields (track, int32 centre on the input grid, radius).
+  Detector._get_additional_inputs splats these on the host; DeviceTracker.init_track hands them to ct_render_tracks."""
+  for trk in dets:
+    if trk['active'] == 0 or trk['score'] < pre_thresh:
+      continue
+    x0, y0, x1, y1 = trans_bbox(trk['bbox'], trans_input, inp_w, inp_h)
+    if not (y1 - y0 > 0 and x1 - x0 > 0):
+      continue
+    radius = max(0, int(gaussian_radius((math.ceil(y1 - y0), math.ceil(x1 - x0)))))
+    centre = np.array([(x0 + x1) / 2, (y0 + y1) / 2], dtype=np.float32)
+    yield trk, centre.astype(np.int32), radius
+
+
 def _round_up(v, m):
   return (v + m - 1) // m * m
 
@@ -256,9 +278,7 @@ class Detector(object):
 
   def _trans_bbox(self, bbox, trans, width, height):
     """Box corners through a 2x3 affine map, clipped to [0, width-1] x [0, height-1] (detector.py:242-251)."""
-    corners = np.asarray(bbox, dtype=np.float32).reshape(2, 2)
-    moved = np.stack([affine_transform(corners[0], trans), affine_transform(corners[1], trans)]).astype(np.float32)
-    return np.clip(moved, 0, np.array([width - 1, height - 1], dtype=np.float32)).reshape(4)
+    return trans_bbox(bbox, trans, width, height)
 
   def _get_additional_inputs(self, dets, meta, with_hm=True):
     """detector.py:254-290: the prior heat-map [1,1,inp_h,inp_w] splatted from the tracks that are active and score at
@@ -266,16 +286,9 @@ class Detector(object):
     inp_w, inp_h, out_w, out_h = meta['inp_width'], meta['inp_height'], meta['out_width'], meta['out_height']
     canvas = np.zeros((1, inp_h, inp_w), dtype=np.float32)
     inds = []
-    for trk in dets:
-      if trk['active'] == 0 or trk['score'] < self.opt.pre_thresh:
-        continue
-      x0, y0, x1, y1 = self._trans_bbox(trk['bbox'], meta['trans_input'], inp_w, inp_h)
-      if not (y1 - y0 > 0 and x1 - x0 > 0):
-        continue
+    for trk, centre, radius in prior_splats(dets, meta['trans_input'], inp_w, inp_h, self.opt.pre_thresh):
       if with_hm:
-        radius = max(0, int(gaussian_radius((math.ceil(y1 - y0), math.ceil(x1 - x0)))))
-        centre = np.array([(x0 + x1) / 2, (y0 + y1) / 2], dtype=np.float32)
-        draw_umich_gaussian(canvas[0], centre.astype(np.int32), radius)
+        draw_umich_gaussian(canvas[0], centre, radius)
       ox0, oy0, ox1, oy1 = self._trans_bbox(trk['bbox'], meta['trans_output'], out_w, out_h)
       cell = np.array([(ox0 + ox1) / 2, (oy0 + oy1) / 2], dtype=np.int32)
       inds.append(cell[1] * out_w + cell[0])

@@ -17,7 +17,10 @@ Two ways to feed the prior heat-map (`--pre_hm`):
   * device_tracking=True (SURVEY 8f-1): the reference's dependency chain closed ON THE DEVICE, inside the same graph:
         pre_hm(t) = splat(tracks(t-1))  ->  network + decode -> records(t)  ->  tracks(t) = Tracker.step(records(t))
     (`DeviceTracker`: ct_render_tracks, ct_track_step).  Exact reference semantics (no stale prior), no host round
-    trip; the host uploads only the frame and downloads the track table (ids, boxes, ages).
+    trip; the host uploads only the frame and downloads the track table (ids, boxes, ages).  Greedy, --hungarian and
+    --public_det association all run in the graph.  With --public_det each input slot also has its own buffer of
+    public detections (the reference's `cur_dets`), uploaded with that slot's frame and read by that slot's graph;
+    `reset_tracking(pre_dets)` seeds every stream's tracker at t = 0 like Tracker.init_track(meta['pre_dets']).
 
 The end-to-end form (`step_host`) takes HOST frames: pinned staging, H2D on a copy stream overlapped
 with the previous step's compute, graph replay, D2H of the records (and tracks).
@@ -36,7 +39,7 @@ NS = 3          # input slots
 class StreamRunner(object):
 
   def __init__(self, model, B, H, W, K=100, precision='bf16', device='cuda', use_graph=True, opt=None,
-               device_tracking=False):
+               device_tracking=False, max_public=None):
     self.B, self.H, self.W, self.K = B, H, W, K
     self.device = torch.device(device)
     self.model = model
@@ -61,9 +64,14 @@ class StreamRunner(object):
     self.tracker = None
     self.device_tracking = device_tracking
     self._eager(0, first=True)                               # sizes the record buffer
+    self.pub = self.h_pub = None
     if device_tracking:
       assert self.opt is not None, 'device tracking needs opt (thresholds, max_age)'
-      self.tracker = DeviceTracker(self.opt, B, K, self.rec.shape[2], self.layout, H, W, self.device)
+      self.tracker = DeviceTracker(self.opt, B, K, self.rec.shape[2], self.layout, H, W, self.device,
+                                   max_public=max_public)
+      if self.tracker.public_det:                            # per slot: public detections of that slot's frame
+        self.pub = [self.tracker.new_public_buffers(self.device) for _ in range(NS)]
+        self.h_pub = [self.tracker.new_public_buffers('cpu', pin=True) for _ in range(NS)]
     torch.cuda.synchronize(self.device)
     self.h_rec = [torch.zeros_like(self.rec, device='cpu').pin_memory() for _ in range(2)]
     if self.tracker is not None:
@@ -87,7 +95,7 @@ class StreamRunner(object):
     if self.rec is None:
       self.rec, self.layout = res.records, res.layout
     if self.tracker is not None:
-      self.tracker.step(self.rec)                            # tracks(t)
+      self.tracker.step(self.rec, None if self.pub is None else self.pub[slot])     # tracks(t)
     return res
 
   def _graph(self, slot):
@@ -118,15 +126,28 @@ class StreamRunner(object):
       self.tracker.reset()
     torch.cuda.synchronize(self.device)
 
-  def reset_tracking(self):
+  def reset_tracking(self, pre_dets=None):
+    """Restarts every stream at t = 0; pre_dets (a list of detection dicts per stream, device_tracking) seeds the
+    trackers as Tracker.init_track does on the first frame of a --public_det video."""
     self.t = 0
     if self.tracker is not None:
       self.tracker.reset()
+      if pre_dets is not None:
+        self.tracker.init_track(pre_dets)
 
-  def load_device_inputs(self, images, pre_hms, slot):
+  def load_device_inputs(self, images, pre_hms, slot, public=None):
+    """public (--public_det): device (centres [B,P,2] fp32, counts [B] int32) of this slot's frame, P <= max_public."""
     self.img[slot].copy_(images)
     if pre_hms is not None:
       self.hm[slot].copy_(pre_hms)
+    if public is not None:
+      centres, counts = public
+      if self.pub is None:
+        raise ValueError('public detections need device_tracking with --public_det')
+      if centres.shape[1] > self.tracker.max_public or int(counts.max()) > self.tracker.max_public:
+        raise ValueError('more public detections than max_public = %d' % self.tracker.max_public)
+      self.pub[slot][0][:, :centres.shape[1]].copy_(centres)
+      self.pub[slot][1].copy_(counts)
 
   def _launch(self, slot):
     if self.t == 0:
@@ -143,11 +164,19 @@ class StreamRunner(object):
     self.t += 1
     return self.rec
 
-  def step_host(self, images, pre_hms=None):
+  def step_host(self, images, pre_hms=None, public_dets=None):
     """images [B,3,H,W] (and pre_hms [B,1,H,W] unless device_tracking): float32 HOST tensors (what
-    Detector.pre_process / _get_additional_inputs produce).  Returns the records of the PREVIOUS call (None the first
-    time) -- a one-step software pipeline: this step's H2D overlaps the previous step's compute."""
+    Detector.pre_process / _get_additional_inputs produce).  public_dets (device_tracking with --public_det): this
+    frame's public detections, a list per stream of dicts with 'ct' (the reference's meta['cur_dets']); None = none.
+    Returns the records of the PREVIOUS call (None the first time) -- a one-step software pipeline: this step's H2D
+    overlaps the previous step's compute."""
     slot = self.t % NS
+    if self.pub is not None:                         # staged on the host now, uploaded with the frame below
+      h_pub, h_cnt = self.h_pub[slot]
+      h_cnt.zero_()
+      self.tracker.fill_public(h_pub, h_cnt, None, public_dets if public_dets is not None else [[]] * self.B)
+    elif public_dets is not None:
+      raise ValueError('public detections need device_tracking with --public_det')
     use_hm = self.tracker is None and pre_hms is not None
     src_img, src_hm = images, pre_hms
     if not images.is_pinned() or (use_hm and not pre_hms.is_pinned()):   # pageable input: stage through pinned memory
@@ -161,6 +190,9 @@ class StreamRunner(object):
       self.img[slot].copy_(src_img, non_blocking=True)
       if use_hm:
         self.hm[slot].copy_(src_hm, non_blocking=True)
+      if self.pub is not None:
+        self.pub[slot][0].copy_(self.h_pub[slot][0], non_blocking=True)
+        self.pub[slot][1].copy_(self.h_pub[slot][1], non_blocking=True)
       self.ev_in[slot].record(self.copy)
     prev = self.fetch() if self.t > 0 else None
     with torch.cuda.stream(self.compute):
@@ -191,7 +223,8 @@ class StreamRunner(object):
 
   @property
   def h2d_bytes_per_step(self):
-    return self.B * (3 if self.tracker is not None else 4) * self.H * self.W * 4
+    pub = 0 if self.pub is None else self.pub[0][0].numel() * 4 + self.pub[0][1].numel() * 4
+    return self.B * (3 if self.tracker is not None else 4) * self.H * self.W * 4 + pub
 
   @property
   def d2h_bytes_per_step(self):

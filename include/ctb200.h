@@ -18,9 +18,10 @@
  *                     + generic_decode, utils.py:16-26,52-87 and decode.py:83-182
  *                     (+ _update_kps_with_hm decode.py:11-81 for the pose heads).
  *   ct_render_pre_hm  Detector._get_additional_inputs's gaussian splat, detector.py:254-290.
- *   ct_track_step     generic_post_process's affine (utils/post_process.py:21-91) + Tracker.step's greedy association
- *                     (utils/tracker.py:28-138) + the (centre, radius) boxes of _get_additional_inputs for the next
- *                     frame, per stream, on the device;  ct_render_tracks splats those boxes (image.py:128-154).
+ *   ct_track_step     generic_post_process's affine (utils/post_process.py:21-91) + Tracker.step's association
+ *                     (utils/tracker.py:28-138: greedy, --hungarian, --public_det births) + the (centre, radius) boxes
+ *                     of _get_additional_inputs for the next frame, per stream, on the device;  ct_render_tracks
+ *                     splats those boxes (image.py:128-154).
  *   ct_flip_merge     Detector._flip_output, detector.py:311-332 (flip_tensor / flip_lr / flip_lr_off, model/utils.py:28-50).
  *   ct_warp_affine_normalize   Detector.pre_process's cv2.warpAffine + normalise + HWC->CHW, detector.py:207-226.
  */
@@ -245,8 +246,24 @@ typedef struct {
   float* tracks;              /* in/out [B,T,CT_TRK_FLOATS]: the stream's tracks == the results of this step */
   int32_t* counts;            /* in/out [B,2]: number of tracks, id_count */
   float* boxes;               /* out [B,T,5] rows (b, cx, cy, radius, 0) for ct_render_tracks, radius < 0 = skip; or NULL */
+  /* Association mode (a zeroed tail = greedy matching, private births: the behaviour before these fields existed). */
+  int32_t assign;             /* ct_track_assign */
+  const float* public_det;    /* [B,max_public,2] image-coordinate centres of the public detections (MOT --public_det,
+                                 tracker.py:83-103): a track may only start on a detection one of them claims; or NULL */
+  const int32_t* public_count; /* [B] public detections of this frame per stream (clamped to max_public); needed with
+                                  public_det */
+  int32_t max_public;         /* row capacity of public_det per stream (>= 0) */
 } ct_track_desc;
 
+typedef enum {
+  CT_ASSIGN_GREEDY = 0,       /* tracker.py:129-138: detections in score order take their nearest free track */
+  CT_ASSIGN_HUNGARIAN = 1     /* --hungarian, tracker.py:52-72: minimum-cost assignment, pair for pair what scipy's
+                                 linear_sum_assignment returns on the gated float64 cost (blocked pairs = 1e18); pairs
+                                 forced through a blocked cell are handed back as unmatched */
+} ct_track_assign;
+
+/* Dynamic shared memory of the largest ct_track_step launch for (K, max_tracks): the track table, this frame's
+ * detections and, for CT_ASSIGN_HUNGARIAN / public_det, the solver's per-column and per-row scratch. */
 int64_t ct_track_smem_bytes(int32_t K, int32_t max_tracks);
 int ct_track_step(const ct_track_desc* d, void* stream);
 /* pre_hm (fp32 [B,1,H,W], zeroed here) <- max-splat of boxes [n,5] (rows with radius < 0 skipped); n is the grid size,
