@@ -4,6 +4,7 @@ The product path has NO CPU fallback: if the library cannot be loaded, or a call
 RuntimeError is raised with ct_last_error().
 """
 import ctypes as C
+import glob
 import os
 import subprocess
 
@@ -86,8 +87,7 @@ NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', 
 def build(force=False, verbose=False):
   """Compile libctb200.so in-tree for sm_100a (nvcc cross-compiles without a GPU)."""
   srcs = [os.path.join(CSRC, s) for s in SOURCES]
-  deps = srcs + [os.path.join(CSRC, h) for h in ('common.cuh', 'conv_common.cuh')] + \
-      [os.path.join(_HERE, '..', 'include', 'ctb200.h')]
+  deps = srcs + glob.glob(os.path.join(CSRC, '*.cuh')) + [os.path.join(_HERE, '..', 'include', 'ctb200.h')]
   if not force and os.path.exists(LIB_PATH) and \
       all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(d) for d in deps):
     return LIB_PATH

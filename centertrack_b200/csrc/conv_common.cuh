@@ -1,7 +1,10 @@
-// Device-side pieces shared by the SIMT (fp32-exact) and tcgen05 (bf16) implicit-GEMM engines:
-// output-pixel decomposition, conv window addressing and DCNv2 bilinear sampling.
+// Pieces shared by the SIMT (fp32-exact) and tcgen05 (bf16) implicit-GEMM engines: output-pixel decomposition, conv
+// window addressing, DCNv2 bilinear sampling, and the tensor-core engines' host-side launch setup.
 #pragma once
 #include "common.cuh"
+#include <cuda.h>
+#include <utility>
+#include <vector>
 
 namespace ctb {
 
@@ -64,10 +67,69 @@ __device__ __forceinline__ float head_transform(float v, int head_act, float dep
   return v;
 }
 
-// cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda at link time)
-typedef int (*TmapEncodeFnRaw)(void*, int, unsigned, void*, const unsigned long long*, const unsigned long long*,
-                               const unsigned*, const unsigned*, int, int, int, int);
-void* tmap_encode_raw();
+// ---- host-side launch setup shared by the tensor-core engines ----
+// cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda at link time); nullptr if unavailable
+typedef CUresult (*TmapEncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                      const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                      CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+inline TmapEncodeTiledFn tmap_encode_tiled() {
+  static TmapEncodeTiledFn fn = nullptr;
+  if (!fn) {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+        q == cudaDriverEntryPointSuccess)
+      fn = reinterpret_cast<TmapEncodeTiledFn>(p);
+  }
+  return fn;
+}
+
+// Tensor map of a bf16 tensor (innermost dimension first, byte strides of the outer ones), unit element strides,
+// zero fill outside the tensor.  `who` names the caller in the error message.
+inline int encode_tmap_bf16(CUtensorMap* map, const void* x, cuuint32_t rank, const cuuint64_t* dims,
+                            const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swizzle,
+                            const char* who) {
+  const TmapEncodeTiledFn enc = tmap_encode_tiled();
+  if (!enc) return fail(CT_ERR_CUDA, "%s: cuTensorMapEncodeTiled entry point unavailable", who);
+  const cuuint32_t estr[4] = {1, 1, 1, 1};
+  const CUresult cr = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, const_cast<void*>(x), dims, strides, box, estr,
+                          CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  return cr == CUDA_SUCCESS ? CT_OK : fail(CT_ERR_CUDA, "%s: cuTensorMapEncodeTiled failed (%ld)", who, (long)cr);
+}
+
+// 4-D map {C, W, H, B} of a bf16 NHWC tensor whose pixel stride is `ld` elements; box {box_c, box_w, box_h, 1}
+inline int encode_tmap_nhwc_bf16(CUtensorMap* map, const void* x, int B, int H, int W, int C, int ld, int box_c,
+                                 int box_w, int box_h, CUtensorMapSwizzle swizzle, const char* who) {
+  const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
+  const cuuint64_t strides[3] = {(cuuint64_t)ld * 2, (cuuint64_t)W * ld * 2, (cuuint64_t)H * W * ld * 2};
+  const cuuint32_t box[4] = {(cuuint32_t)box_c, (cuuint32_t)box_w, (cuuint32_t)box_h, 1};
+  return encode_tmap_bf16(map, x, 4, dims, strides, box, swizzle, who);
+}
+
+// Raises `kernel`'s dynamic shared-memory limit to `bytes`, once per (kernel, device): the attribute is per device, and
+// a process may drive several GPUs from one thread.
+inline cudaError_t set_max_dynamic_smem_once(const void* kernel, int bytes) {
+  int dev = 0;
+  cudaGetDevice(&dev);
+  static thread_local std::vector<std::pair<const void*, int>> done;
+  for (const auto& e : done)
+    if (e.first == kernel && e.second == dev) return cudaSuccess;
+  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e == cudaSuccess) done.emplace_back(kernel, dev);
+  return e;
+}
+
+// SM count of the current device, queried once per device (148 if the query fails)
+inline int sm_count() {
+  int dev = 0;
+  cudaGetDevice(&dev);
+  static thread_local std::vector<int> sms;
+  if ((int)sms.size() <= dev) sms.resize(dev + 1, 0);
+  if (sms[dev] == 0 && cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+    sms[dev] = 0;
+  return sms[dev] > 0 ? sms[dev] : 148;
+}
 
 int conv_forward_simt(const ct_conv_desc* d, cudaStream_t st);
 int conv_forward_tc(const ct_conv_desc* d, cudaStream_t st);

@@ -19,8 +19,7 @@
 // (two per SM sub-partition) because the gather is latency-bound: more warps = more loads in flight.
 // Two CTAs are co-resident per SM so one CTA's epilogue overlaps another's main loop.
 #include "conv_common.cuh"
-#include <cuda.h>
-#include <stdlib.h>
+#include "sm100.cuh"
 
 namespace ctb {
 
@@ -30,6 +29,9 @@ constexpr int TC_THREADS = 288;        // 8 producer/epilogue warps + 1 MMA warp
 constexpr int TC_PRODUCERS = 256;
 constexpr int TC_NROW = TC_BM * 8 / TC_PRODUCERS;   // A-tile rows per producer thread per K slice (4)
 constexpr int A_STAGE_BYTES = TC_BM * 128;
+// CT_A_DCN_WIN: pixels of offset margin staged around a patch's 3x3 footprint (samples that leave it read global memory).
+// Margins 1 / 2 / 3 measured on B200: 2 is fastest (DESIGN.md).
+constexpr int DCN_WIN_MARGIN = 2;
 
 struct TcArgs {
   ConvGeom g;
@@ -40,13 +42,10 @@ struct TcArgs {
   const float* om;
   void* out;
   int n_tile, k_slices, stages, tmem_cols, a_mode;
-  int tiles_x, tiles_y;         // > 0: an M tile is an 8 (y) x 16 (x) pixel patch of one image (L1 reuse of the
-                                // 3x3 / bilinear footprints); 0: 128 consecutive pixels in b,y,x order
+  int tiles_x, tiles_y;         // CT_A_DCN_WIN: an M tile is an 8 (y) x 16 (x) pixel patch of one image;
+                                // 0: 128 consecutive pixels in b,y,x order
   int win_m, win_pw, win_ph;    // CT_A_DCN_WIN: offset margin (px) and the staged window (pixels) of one 8x16 patch
   uint32_t win_bytes;           // bytes of one 64-channel window (= TMA box)
-  int fence_mma;                // 1: the generic->async proxy fence is executed by the MMA thread after the full-barrier
-                                // wait instead of by every producer (fence.proxy.async compiles to MEMBAR.ALL.CTA +
-                                // FENCE.VIEW.ASYNC, and the MEMBAR drains the producer's prefetched global loads)
 };
 
 // CT_A_DCN_WIN sampling record (16 bytes): global fall-back offset of the clamped top-left corner (channel 0 of the
@@ -61,11 +60,6 @@ __device__ __forceinline__ uint4 lds16(uint32_t addr) {
   uint4 r;
   asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(addr));
   return r;
-}
-__device__ __forceinline__ void tma_4d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, int c3, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
-      ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(bar) : "memory");
 }
 
 // output pixel (linear b,y,x index) of GEMM row r of M tile mt; g.P_out when the row is padding
@@ -92,70 +86,6 @@ __device__ __forceinline__ void tc_stamp(unsigned long long* t, int k) {
   if (t != nullptr && k < 256) t[k] = (unsigned long long)clock64();
 }
 
-// ---------------------------------------------------------------------------------------------
-// PTX wrappers
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0;
-  uint32_t spins = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    if (done) break;
-    if (++spins > 20000000u) __trap();   // watchdog: a protocol bug must not hang the GPU
-  }
-}
-__device__ __forceinline__ void fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-      "l"(src), "r"(bytes), "r"(bar)
-      : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_mma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                       uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
 __device__ __forceinline__ uint4 ldg_nc16(const void* p) {
   uint4 r;
   asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
@@ -163,17 +93,6 @@ __device__ __forceinline__ uint4 ldg_nc16(const void* p) {
 }
 __device__ __forceinline__ void sts16(uint32_t addr, uint4 v) {
   asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-
-// K-major, 128B-swizzled smem operand descriptor (cute::UMMA::SmemDescriptor):
-//   [0,14) start>>4 | [16,30) LBO>>4 (=1, unused for swizzled K-major) | [32,46) SBO>>4 (=64: 8 rows x 128B)
-//   [46,48) version=1 | [61,64) layout = 2 (SWIZZLE_128B)
-__device__ __forceinline__ uint64_t make_sdesc(uint32_t smem_addr) {
-  return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
-}
-// kind::f16 instruction descriptor (cute::UMMA::InstrDescriptor): D=f32, A=B=bf16, K-major both.
-__device__ __forceinline__ uint32_t make_idesc(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
 }
 
 // Per (tap, output pixel) DCNv2 sampling record, built once per CTA: clamped top-left corner as a 32-bit element
@@ -295,21 +214,18 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
   pdl_trigger();                       // the next kernel of the stream may start its own prologue now
 
   if (tid == 0) {
-    for (int s = 0; s < S; ++s) { mbar_init(full_bar(s), TC_PRODUCERS / 32); mbar_init(empty_bar(s), 1); }
-    mbar_init(tmem_full_bar, 1);
-    mbar_init(win_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < S; ++s) { mbarrier_init(full_bar(s), TC_PRODUCERS / 32); mbarrier_init(empty_bar(s), 1); }
+    mbarrier_init(tmem_full_bar, 1);
+    mbarrier_init(win_bar, 1);
+    fence_mbarrier_init();
   }
   if (warp == 8) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     smem_u32((const void*)tmem_slot)),
-                 "r"((uint32_t)a.tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tcgen05_alloc(smem_u32((const void*)tmem_slot), (uint32_t)a.tmem_cols);
+    tcgen05_relinquish_alloc_permit();
   }
-  tc_fence_before();
+  tcgen05_fence_before_thread_sync();
   __syncthreads();
-  tc_fence_after();
+  tcgen05_fence_after_thread_sync();
   const uint32_t tmem_base = *tmem_slot;
   if (tid == 0) tc_stamp(trace, 7);
   pdl_wait();                          // everything below reads what the previous kernel wrote
@@ -325,20 +241,6 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
       // DCN rows come from the sampling table
 #pragma unroll
       for (int i = 0; i < TC_NROW; ++i) { row_off[i] = 0; row_iy[i] = -100000; row_ix[i] = -100000; }
-    } else if (a.tiles_x != 0) {
-#pragma unroll
-      for (int i = 0; i < TC_NROW; ++i) {
-        const int p = tc_pixel(a, mt, r0 + 32 * i);   // DCN rows come from its table
-        if (p < g.P_out) {
-          const int b = p / HWo, r = p - b * HWo;
-          const int oy = r / g.OW, ox = r - oy * g.OW;
-          row_iy[i] = oy * g.stride - g.pad;
-          row_ix[i] = ox * g.stride - g.pad_w;
-          row_off[i] = (b * g.H * g.W + row_iy[i] * g.W + row_ix[i]) * g.ld_in;
-        } else {
-          row_off[i] = 0; row_iy[i] = -100000; row_ix[i] = -100000;
-        }
-      }
     } else {
       // linear tiles: one division pair for the first row, the other rows (+32 pixels each) by carry propagation
       int p = mt * TC_BM + r0;
@@ -369,8 +271,8 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
       win_y0 = ty * 8 - 1 - a.win_m;
       win_x0 = tx * 16 - 1 - a.win_m;
       if (tid == 0) {                                   // first 64-channel chunk of the window: TMA, zero fill outside
-        mbar_arrive_expect_tx(win_bar, a.win_bytes);      // count 1: this arrival + the TMA's bytes complete the phase
-        tma_4d(s_win, &tmap, 0, win_x0, win_y0, win_b, win_bar);
+        mbarrier_arrive_expect_tx(win_bar, a.win_bytes);      // count 1: this arrival + the TMA's bytes complete the phase
+        cp_async_bulk_tensor_4d(s_win, &tmap, 0, win_x0, win_y0, win_b, win_bar);
       }
       // Two threads per row (taps 0-4 and 5-8) so that all eight producer warps build the table.  The 27 offset / mask
       // floats of a row sit in one 128-byte line of `om`; each thread loads only the 16-byte chunks its taps need.
@@ -486,14 +388,14 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
       const int gdx = g.ld_in, gdy = g.W * g.ld_in;
       int s = 0;
       for (int ch = 0; ch < nchunks; ++ch) {
-        mbar_wait(win_bar, (uint32_t)ch & 1u);
+        mbarrier_wait_parity(win_bar, (uint32_t)ch & 1u);
         for (int tap = 0; tap < 9; ++tap, ++s) {
           const int stage = s % S;
           const uint32_t ph = (uint32_t)(s / S) & 1u;
-          mbar_wait(empty_bar(stage), ph ^ 1u);
+          mbarrier_wait_parity(empty_bar(stage), ph ^ 1u);
           if (tid == 0) {
-            mbar_expect_tx(full_bar(stage), b_stage_bytes);
-            bulk_g2s(sB + stage * b_stage_bytes, wt + (size_t)s * w_slice_elems, b_stage_bytes, full_bar(stage));
+            mbarrier_expect_tx(full_bar(stage), b_stage_bytes);
+            cp_async_bulk(sB + stage * b_stage_bytes, wt + (size_t)s * w_slice_elems, b_stage_bytes, full_bar(stage));
           }
           const DcnWinEntry* tab = win_tab + tap * TC_BM + r0;
           uint4 e4[TC_NROW], v[TC_NROW][4];
@@ -526,16 +428,15 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
             o.x = bfma2(v[i][3].x, w3, o.x); o.y = bfma2(v[i][3].y, w3, o.y); o.z = bfma2(v[i][3].z, w3, o.z); o.w = bfma2(v[i][3].w, w3, o.w);
             sts16(dst + i * 4096u, o);
           }
-          if (!a.fence_mma) fence_proxy_async();
           __syncwarp();
-          if (lane == 0) mbar_arrive(full_bar(stage));
+          if (lane == 0) mbarrier_arrive(full_bar(stage));
           if (tid == 0) tc_stamp(trace, 8 + s);
         }
         if (ch + 1 < nchunks) {                       // every producer is done with this chunk's window: refill it
           asm volatile("bar.sync 1, 256;" ::: "memory");
           if (tid == 0) {
-            mbar_arrive_expect_tx(win_bar, a.win_bytes);      // count 1: this arrival + the TMA's bytes complete the phase
-            tma_4d(s_win, &tmap, (ch + 1) << 6, win_x0, win_y0, win_b, win_bar);
+            mbarrier_arrive_expect_tx(win_bar, a.win_bytes);      // count 1: this arrival + the TMA's bytes complete the phase
+            cp_async_bulk_tensor_4d(s_win, &tmap, (ch + 1) << 6, win_x0, win_y0, win_b, win_bar);
           }
         }
       }
@@ -544,17 +445,16 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
       auto begin_stage = [&](int s) {
         const int stage = s % S;
         const uint32_t ph = (uint32_t)(s / S) & 1u;
-        mbar_wait(empty_bar(stage), ph ^ 1u);
+        mbarrier_wait_parity(empty_bar(stage), ph ^ 1u);
         if (tid == 0) {
-          mbar_expect_tx(full_bar(stage), b_stage_bytes);
-          bulk_g2s(sB + stage * b_stage_bytes, wt + (size_t)s * w_slice_elems, b_stage_bytes, full_bar(stage));
+          mbarrier_expect_tx(full_bar(stage), b_stage_bytes);
+          cp_async_bulk(sB + stage * b_stage_bytes, wt + (size_t)s * w_slice_elems, b_stage_bytes, full_bar(stage));
         }
         return stage;
       };
       auto end_stage = [&](int s, int stage) {
-        if (!a.fence_mma) fence_proxy_async();
         __syncwarp();
-        if (lane == 0) mbar_arrive(full_bar(stage));
+        if (lane == 0) mbarrier_arrive(full_bar(stage));
         if (tid == 0) tc_stamp(trace, 8 + s);
       };
       if (a.a_mode == CT_A_DCN) {
@@ -693,10 +593,10 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
         const int stage = s % S;
         const uint32_t ph = (uint32_t)(s / S) & 1u;
         load_half(tap, cq << 3, 1, vb);
-        mbar_wait(empty_bar(stage), ph ^ 1u);
+        mbarrier_wait_parity(empty_bar(stage), ph ^ 1u);
         if (tid == 0) {
-          mbar_expect_tx(full_bar(stage), b_stage_bytes);
-          bulk_g2s(sB + stage * b_stage_bytes, wt + (size_t)s * a.n_tile * TC_BK, b_stage_bytes, full_bar(stage));
+          mbarrier_expect_tx(full_bar(stage), b_stage_bytes);
+          cp_async_bulk(sB + stage * b_stage_bytes, wt + (size_t)s * a.n_tile * TC_BK, b_stage_bytes, full_bar(stage));
         }
         blend_half(tap, stage, 0, va);
         int ntap = tap, ncq = cq + 8;
@@ -704,9 +604,8 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
         if (s + 1 < a.k_slices) load_half(ntap, ncq << 3, 0, va);
         blend_half(tap, stage, 1, vb);
         tap = ntap; cq = ncq;
-        if (!a.fence_mma) fence_proxy_async();
         __syncwarp();
-        if (lane == 0) mbar_arrive(full_bar(stage));      // one arrival per producer warp
+        if (lane == 0) mbarrier_arrive(full_bar(stage));      // one arrival per producer warp
         if (tid == 0) tc_stamp(trace, 8 + s);
       }
     } else {
@@ -731,17 +630,16 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
       auto store_slice = [&](int s, const uint4 (&v)[TC_NROW]) {
         const int stage = s % S;
         const uint32_t ph = (uint32_t)(s / S) & 1u;
-        mbar_wait(empty_bar(stage), ph ^ 1u);
+        mbarrier_wait_parity(empty_bar(stage), ph ^ 1u);
         if (tid == 0) {
-          mbar_expect_tx(full_bar(stage), b_stage_bytes);
-          bulk_g2s(sB + stage * b_stage_bytes, wt + (size_t)s * a.n_tile * TC_BK, b_stage_bytes, full_bar(stage));
+          mbarrier_expect_tx(full_bar(stage), b_stage_bytes);
+          cp_async_bulk(sB + stage * b_stage_bytes, wt + (size_t)s * a.n_tile * TC_BK, b_stage_bytes, full_bar(stage));
         }
         const uint32_t dst = sA + stage * A_STAGE_BYTES + (uint32_t)r0 * 128u + swz;
 #pragma unroll
         for (int i = 0; i < TC_NROW; ++i) sts16(dst + i * 4096u, v[i]);
-        if (!a.fence_mma) fence_proxy_async();          // generic-proxy smem writes -> visible to the tensor-core (async) proxy
         __syncwarp();
-        if (lane == 0) mbar_arrive(full_bar(stage));      // one arrival per producer warp (256 arrivals on one
+        if (lane == 0) mbarrier_arrive(full_bar(stage));      // one arrival per producer warp (256 arrivals on one
                                                           // shared-memory word serialise)
         if (tid == 0) tc_stamp(trace, 8 + s);
       };
@@ -759,8 +657,8 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
     }
 
     // =========================== epilogue ===========================
-    mbar_wait(tmem_full_bar, 0);
-    tc_fence_after();
+    mbarrier_wait_parity(tmem_full_bar, 0);
+    tcgen05_fence_after_thread_sync();
     if (tid == 0) tc_stamp(trace, 5);
     const int wq = warp & 3, chalf = warp >> 2;      // TMEM lane quarter, column-chunk parity
     const int row = wq * 32 + lane;
@@ -769,7 +667,7 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
     const uint32_t t_lane = tmem_base + ((uint32_t)(wq * 32) << 16);
     for (int col = chalf * 16; col < a.n_tile; col += 32) {
       uint32_t r[16];
-      tc_ld16(t_lane + (uint32_t)col, r);
+      tcgen05_ld_32x32b_x16(t_lane + (uint32_t)col, r);
       const int o0 = n0 + col;
       if (!p_ok || o0 >= g.C_out) continue;
       float v[16];
@@ -867,42 +765,43 @@ conv_tc_kernel(const TcArgs a, const __grid_constant__ CUtensorMap tmap) {
     }
   } else if (lane == 0) {
     // =========================== MMA issuer (one thread) ===========================
-    const uint32_t idesc = make_idesc(a.n_tile);
+    const uint32_t idesc = umma_idesc_bf16_m128(a.n_tile);
     for (int s = 0; s < a.k_slices; ++s) {
       const int stage = s % S;
       const uint32_t ph = (uint32_t)(s / S) & 1u;
-      mbar_wait(full_bar(stage), ph);
-      if (a.fence_mma) fence_proxy_async();      // the producers' st.shared (acquired through the barrier) -> async proxy
-      tc_fence_after();
-      const uint64_t ad = make_sdesc(sA + stage * a_stage_bytes);
-      const uint64_t bd = make_sdesc(sB + stage * b_stage_bytes);
+      mbarrier_wait_parity(full_bar(stage), ph);
+      // the producers' st.shared (acquired through the barrier) -> async proxy.  Fenced here rather than by every producer:
+      // fence.proxy.async compiles to MEMBAR.ALL.CTA + FENCE.VIEW.ASYNC, and the MEMBAR drains the producer's prefetched loads
+      fence_proxy_async_shared_cta();
+      tcgen05_fence_after_thread_sync();
+      const uint64_t ad = umma_sdesc_sw128(sA + stage * a_stage_bytes);
+      const uint64_t bd = umma_sdesc_sw128(sB + stage * b_stage_bytes);
       if constexpr (X3) {
-        const uint64_t ad_lo = make_sdesc(sA + stage * a_stage_bytes + A_STAGE_BYTES);
-        const uint64_t bd_lo = make_sdesc(sB + stage * b_stage_bytes + b_tile_bytes);
+        const uint64_t ad_lo = umma_sdesc_sw128(sA + stage * a_stage_bytes + A_STAGE_BYTES);
+        const uint64_t bd_lo = umma_sdesc_sw128(sB + stage * b_stage_bytes + b_tile_bytes);
 #pragma unroll
         for (int k = 0; k < TC_BK / 16; ++k) {      // small cross terms first, then the hi x hi term
-          tc_mma(tmem_base, ad_lo + 2ull * k, bd + 2ull * k, idesc, (s > 0 || k > 0) ? 1u : 0u);
-          tc_mma(tmem_base, ad + 2ull * k, bd_lo + 2ull * k, idesc, 1u);
-          tc_mma(tmem_base, ad + 2ull * k, bd + 2ull * k, idesc, 1u);
+          tcgen05_mma(tmem_base, ad_lo + 2ull * k, bd + 2ull * k, idesc, (s > 0 || k > 0) ? 1u : 0u);
+          tcgen05_mma(tmem_base, ad + 2ull * k, bd_lo + 2ull * k, idesc, 1u);
+          tcgen05_mma(tmem_base, ad + 2ull * k, bd + 2ull * k, idesc, 1u);
         }
       } else {
 #pragma unroll
         for (int k = 0; k < TC_BK / 16; ++k)
-          tc_mma(tmem_base, ad + 2ull * k, bd + 2ull * k, idesc, (s > 0 || k > 0) ? 1u : 0u);
+          tcgen05_mma(tmem_base, ad + 2ull * k, bd + 2ull * k, idesc, (s > 0 || k > 0) ? 1u : 0u);
       }
-      tc_commit(empty_bar(stage));     // frees this smem stage when the MMAs above have read it
+      tcgen05_commit(empty_bar(stage));     // frees this smem stage when the MMAs above have read it
     }
-    tc_commit(tmem_full_bar);           // accumulator complete -> epilogue
+    tcgen05_commit(tmem_full_bar);           // accumulator complete -> epilogue
     tc_stamp(trace, 4);
   }
 
-  tc_fence_before();
+  tcgen05_fence_before_thread_sync();
   __syncthreads();
   if (tid == 0) tc_stamp(trace, 6);
   if (warp == 8) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)a.tmem_cols)
-                 : "memory");
+    tcgen05_fence_after_thread_sync();
+    tcgen05_dealloc(tmem_base, (uint32_t)a.tmem_cols);
   }
 }
 
@@ -968,21 +867,20 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
 
   pdl_trigger();
   if (tid == 0) {
-    for (int s = 0; s < DP_SA; ++s) { mbar_init(full_bar(s), DP_PWARPS + 1); mbar_init(empty_bar(s), 1); }   // 16 producer warps + the TMA warp's expect_tx arrival
+    for (int s = 0; s < DP_SA; ++s) { mbarrier_init(full_bar(s), DP_PWARPS + 1); mbarrier_init(empty_bar(s), 1); }   // 16 producer warps + the TMA warp's expect_tx arrival
     for (int i = 0; i < 2; ++i) {
-      mbar_init(win_full(i), 1); mbar_init(acc_full(i), 1); mbar_init(acc_empty(i), 4); mbar_init(win_empty(i), DP_PWARPS);
-      mbar_init(tab_full(i), 4); mbar_init(tab_empty(i), DP_PWARPS);
+      mbarrier_init(win_full(i), 1); mbarrier_init(acc_full(i), 1); mbarrier_init(acc_empty(i), 4); mbarrier_init(win_empty(i), DP_PWARPS);
+      mbarrier_init(tab_full(i), 4); mbarrier_init(tab_empty(i), DP_PWARPS);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   if (warp == DP_PWARPS) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void*)tmem_slot)),
-                 "r"((uint32_t)a.tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tcgen05_alloc(smem_u32((const void*)tmem_slot), (uint32_t)a.tmem_cols);
+    tcgen05_relinquish_alloc_permit();
   }
-  tc_fence_before();
+  tcgen05_fence_before_thread_sync();
   __syncthreads();
-  tc_fence_after();
+  tcgen05_fence_after_thread_sync();
   const uint32_t tmem_base = *tmem_slot;
   pdl_wait();
 
@@ -1005,15 +903,15 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
     int s = 0;
     for (int t = 0; t < n_my; ++t) {
       const DcnWinEntry* tab_cur = tabs + (t & 1) * 9 * TC_BM;
-      mbar_wait(tab_full(t & 1), (uint32_t)(t >> 1) & 1u);
+      mbarrier_wait_parity(tab_full(t & 1), (uint32_t)(t >> 1) & 1u);
       for (int ch = 0; ch < nchunks; ++ch) {
         const int u = t * nchunks + ch;
         const uint32_t s_win = sWin + (uint32_t)(u & 1) * win_stride;
-        mbar_wait(win_full(u & 1), (uint32_t)(u >> 1) & 1u);
+        mbarrier_wait_parity(win_full(u & 1), (uint32_t)(u >> 1) & 1u);
         for (int tap = 0; tap < 9; ++tap, ++s) {
           const int stage = s % DP_SA;
           const uint32_t ph = (uint32_t)(s / DP_SA) & 1u;
-          mbar_wait(empty_bar(stage), ph ^ 1u);
+          mbarrier_wait_parity(empty_bar(stage), ph ^ 1u);
           if (tid == 0 && s < 60) tc_stamp(trace, 16 + 4 * s);
           const DcnWinEntry* tab = tab_cur + tap * TC_BM + r0;
           uint4 e4[DP_NROW], v[DP_NROW][4];
@@ -1046,14 +944,13 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
             o.x = bfma2(v[i][3].x, w3, o.x); o.y = bfma2(v[i][3].y, w3, o.y); o.z = bfma2(v[i][3].z, w3, o.z); o.w = bfma2(v[i][3].w, w3, o.w);
             sts16(dst + i * 8192u, o);
           }
-          if (!a.fence_mma) fence_proxy_async();
           __syncwarp();
-          if (lane == 0) mbar_arrive(full_bar(stage));
+          if (lane == 0) mbarrier_arrive(full_bar(stage));
           if (tid == 0 && s < 60) tc_stamp(trace, 16 + 4 * s + 1);
         }
-        if (lane == 0) mbar_arrive(win_empty(u & 1));                    // this warp is done with the unit's window
+        if (lane == 0) mbarrier_arrive(win_empty(u & 1));                    // this warp is done with the unit's window
       }
-      if (lane == 0) mbar_arrive(tab_empty(t & 1));                      // ... and with the tile's table
+      if (lane == 0) mbarrier_arrive(tab_empty(t & 1));                      // ... and with the tile's table
     }
   } else if (warp >= DP_PWARPS + 6) {
     // ======================================= table warps: one thread per A-tile row =======================================
@@ -1079,7 +976,7 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
           omv[4 * j] = f.x; omv[4 * j + 1] = f.y; omv[4 * j + 2] = f.z; omv[4 * j + 3] = f.w;
         }
       }
-      if (t >= 2) mbar_wait(tab_empty(t & 1), (uint32_t)((t - 2) >> 1) & 1u);
+      if (t >= 2) mbarrier_wait_parity(tab_empty(t & 1), (uint32_t)((t - 2) >> 1) & 1u);
       DcnWinEntry* tab = tabs + (t & 1) * 9 * TC_BM + trow;
 #pragma unroll
       for (int tap = 0; tap < 9; ++tap) {
@@ -1109,7 +1006,7 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
         tab[tap * TC_BM] = e;
       }
       __syncwarp();
-      if (lane == 0) mbar_arrive(tab_full(t & 1));
+      if (lane == 0) mbarrier_arrive(tab_full(t & 1));
     }
   } else if (warp == DP_PWARPS + 5) {
     // ======================================= TMA issuer =======================================
@@ -1119,10 +1016,10 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
       const int t = u / nchunks, ch = u - t * nchunks;
       int b, ty, tx;
       dp_tile_origin(a, (int)blockIdx.x + t * G, b, ty, tx);
-      if (ry0 == 0) mbar_arrive_expect_tx(win_full(u & 1), a.win_bytes);
+      if (ry0 == 0) mbarrier_arrive_expect_tx(win_full(u & 1), a.win_bytes);
       const uint32_t row_bytes = (uint32_t)a.win_pw * 128u;
       for (int ry = ry0; ry < ry1 && ry < a.win_ph; ++ry)
-        tma_4d(sWin + (uint32_t)(u & 1) * win_stride + (uint32_t)ry * row_bytes, &tmap, ch << 6, tx * 16 - 1 - a.win_m,
+        cp_async_bulk_tensor_4d(sWin + (uint32_t)(u & 1) * win_stride + (uint32_t)ry * row_bytes, &tmap, ch << 6, tx * 16 - 1 - a.win_m,
                ty * 8 - 1 - a.win_m + ry, b, win_full(u & 1));
     };
       issue_window_rows(0, 0, a.win_ph);
@@ -1132,15 +1029,15 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
         for (int tap = 0; tap < 9; ++tap, ++s) {
           const int stage = s % DP_SA;
           const uint32_t ph = (uint32_t)(s / DP_SA) & 1u;
-          mbar_wait(empty_bar(stage), ph ^ 1u);
-          mbar_arrive_expect_tx(full_bar(stage), b_tile_bytes);        // the weight tile first: the MMA of this slice waits for it
-          bulk_g2s(sB + stage * b_tile_bytes, a.w + (size_t)(ch * 9 + tap) * a.n_tile * TC_BK, b_tile_bytes, full_bar(stage));
+          mbarrier_wait_parity(empty_bar(stage), ph ^ 1u);
+          mbarrier_arrive_expect_tx(full_bar(stage), b_tile_bytes);        // the weight tile first: the MMA of this slice waits for it
+          cp_async_bulk(sB + stage * b_tile_bytes, a.w + (size_t)(ch * 9 + tap) * a.n_tile * TC_BK, b_tile_bytes, full_bar(stage));
           // next unit's window into the other buffer, three rows per slice from tap 3 on: issuing a request costs this
           // thread ~100+ cycles, and 15 of them ahead of the first weight tiles of a unit stalled every tile boundary by
           // ~4000 cycles.  This warp runs at most DP_SA slices ahead of the producers, so by tap 3 they have released
           // the buffer (unit u - 1) and the wait below does not block.
           if (u + 1 < n_units && tap >= 3) {
-            if (tap == 3 && u >= 1) mbar_wait(win_empty((u + 1) & 1), (uint32_t)((u - 1) >> 1) & 1u);
+            if (tap == 3 && u >= 1) mbarrier_wait_parity(win_empty((u + 1) & 1), (uint32_t)((u - 1) >> 1) & 1u);
             issue_window_rows(u + 1, 3 * (tap - 3), 3 * (tap - 3) + 3);
           }
         }
@@ -1149,29 +1046,29 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
   } else if (warp == DP_PWARPS) {
     // ======================================= MMA issuer =======================================
     if (lane == 0) {
-      const uint32_t idesc = make_idesc(a.n_tile);
+      const uint32_t idesc = umma_idesc_bf16_m128(a.n_tile);
       int s = 0;
       for (int t = 0; t < n_my; ++t) {
         const int ai = t & 1;
-        mbar_wait(acc_empty(ai), ((uint32_t)(t >> 1) & 1u) ^ 1u);
-        tc_fence_after();
+        mbarrier_wait_parity(acc_empty(ai), ((uint32_t)(t >> 1) & 1u) ^ 1u);
+        tcgen05_fence_after_thread_sync();
         const uint32_t d_tmem = tmem_base + (uint32_t)(ai * a.n_tile);
         for (int sl = 0; sl < 9 * nchunks; ++sl, ++s) {
           const int stage = s % DP_SA;
           const uint32_t ph = (uint32_t)(s / DP_SA) & 1u;
-          mbar_wait(full_bar(stage), ph);
-          if (a.fence_mma) fence_proxy_async();
-          tc_fence_after();
+          mbarrier_wait_parity(full_bar(stage), ph);
+          fence_proxy_async_shared_cta();
+          tcgen05_fence_after_thread_sync();
           if (s < 60) tc_stamp(trace, 16 + 4 * s + 2);
-          const uint64_t ad = make_sdesc(sA + stage * A_STAGE_BYTES);
-          const uint64_t bd = make_sdesc(sB + stage * b_tile_bytes);
+          const uint64_t ad = umma_sdesc_sw128(sA + stage * A_STAGE_BYTES);
+          const uint64_t bd = umma_sdesc_sw128(sB + stage * b_tile_bytes);
 #pragma unroll
           for (int k = 0; k < TC_BK / 16; ++k)
-            tc_mma(d_tmem, ad + 2ull * k, bd + 2ull * k, idesc, (sl > 0 || k > 0) ? 1u : 0u);
-          tc_commit(empty_bar(stage));
+            tcgen05_mma(d_tmem, ad + 2ull * k, bd + 2ull * k, idesc, (sl > 0 || k > 0) ? 1u : 0u);
+          tcgen05_commit(empty_bar(stage));
           if (s < 60) tc_stamp(trace, 16 + 4 * s + 3);
         }
-        tc_commit(acc_full(ai));
+        tcgen05_commit(acc_full(ai));
       }
     }
   } else {
@@ -1185,12 +1082,12 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
       const int oy = ty * 8 + (row >> 4), ox = tx * 16 + (row & 15);
       const bool p_ok = oy < g.OH && ox < g.OW;
       const size_t p = ((size_t)b * g.OH + oy) * g.OW + ox;
-      mbar_wait(acc_full(ai), (uint32_t)(t >> 1) & 1u);
-      tc_fence_after();
+      mbarrier_wait_parity(acc_full(ai), (uint32_t)(t >> 1) & 1u);
+      tcgen05_fence_after_thread_sync();
       const uint32_t t_lane = tmem_base + ((uint32_t)(wq * 32) << 16) + (uint32_t)(ai * a.n_tile);
       for (int col = 0; col < a.n_tile; col += 16) {
         uint32_t r[16];
-        tc_ld16(t_lane + (uint32_t)col, r);
+        tcgen05_ld_32x32b_x16(t_lane + (uint32_t)col, r);
         if (!p_ok || col >= g.C_out) continue;
         float v[16];
 #pragma unroll
@@ -1218,24 +1115,19 @@ dcn_persist_kernel(const TcArgs a, const int tiles_total, const __grid_constant_
         uint4* op = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(a.out) + p * g.ld_out + col);
         op[0] = oa; op[1] = ob;
       }
-      tc_fence_before();
+      tcgen05_fence_before_thread_sync();
       __syncwarp();
-      if (lane == 0) mbar_arrive(acc_empty(ai));
+      if (lane == 0) mbarrier_arrive(acc_empty(ai));
     }
   }
 
-  tc_fence_before();
+  tcgen05_fence_before_thread_sync();
   __syncthreads();
   if (warp == DP_PWARPS) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)a.tmem_cols) : "memory");
+    tcgen05_fence_after_thread_sync();
+    tcgen05_dealloc(tmem_base, (uint32_t)a.tmem_cols);
   }
 }
-
-typedef CUresult (*TmapEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                 const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                 CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static TmapEncodeFn tmap_encode_fn() { return reinterpret_cast<TmapEncodeFn>(tmap_encode_raw()); }
 
 int tc_set_trace(void* buf) {
   unsigned long long* p = (unsigned long long*)buf;
@@ -1246,8 +1138,6 @@ int conv_forward_tc(const ct_conv_desc* d, cudaStream_t st) {
   const bool x3 = d->engine == CT_ENGINE_TCGEN05_X3;     // fp32 activations, bf16 hi/lo split operands
   TcArgs a;
   a.g = make_geom(d);
-  static const int fence_mma_env = getenv("CTB_TC_FENCE_MMA") ? atoi(getenv("CTB_TC_FENCE_MMA")) : 1;
-  a.fence_mma = fence_mma_env;
   const ConvGeom& g = a.g;
   if (g.C_in % 8 != 0 || g.ld_in % 8 != 0)
     return fail(CT_ERR_INVALID, "conv_tc: C_in and ld_in must be multiples of 8%s (%ld,%ld)", "", g.C_in, g.ld_in);
@@ -1282,8 +1172,7 @@ int conv_forward_tc(const ct_conv_desc* d, cudaStream_t st) {
   const bool win = d->a_mode == CT_A_DCN_WIN;
   if (win && (x3 || g.C_in % 64 != 0))
     return fail(CT_ERR_INVALID, "conv_tc: CT_A_DCN_WIN needs the bf16 engine and C_in %% 64 == 0%s (%ld)", "", g.C_in);
-  static const int win_margin = getenv("CTB_TC_DCN_MARGIN") ? atoi(getenv("CTB_TC_DCN_MARGIN")) : 2;
-  a.win_m = win_margin < 0 ? 0 : (win_margin > 6 ? 6 : win_margin);
+  a.win_m = DCN_WIN_MARGIN;
   a.win_pw = 16 + 2 * a.win_m + 3;
   a.win_ph = 8 + 2 * a.win_m + 3;
   a.win_bytes = (uint32_t)(a.win_pw * a.win_ph * 128);
@@ -1301,18 +1190,15 @@ int conv_forward_tc(const ct_conv_desc* d, cudaStream_t st) {
   if (d->a_mode == CT_A_DCN) {
     // the DCN gather, not the MMA, paces the pipeline: fewer stages leave more of the SM's 228 KB to L1, which
     // the bilinear corner reads (each input pixel is touched ~36 times) depend on
-    static const int dcn_stages = getenv("CTB_TC_DCN_STAGES") ? atoi(getenv("CTB_TC_DCN_STAGES")) : 2;
-    if (dcn_stages >= 2 && dcn_stages < stages) stages = dcn_stages;
+    stages = 2;
   }
   if (win) {
     // two CTAs per SM: table 18 KB + window 43 KB + stages x (16 KB + n_tile x 128 B) must stay under ~113 KB
-    static const int win_stages = getenv("CTB_TC_WIN_STAGES") ? atoi(getenv("CTB_TC_WIN_STAGES")) : 0;
     stages = 2;
     if (smem_for(2) > 113 * 1024) {                  // one CTA per SM anyway (wide N tile): deepen the pipeline instead
       stages = 4;
       while (stages > 2 && smem_for(stages) > 200 * 1024) --stages;
     }
-    if (win_stages >= 2) stages = win_stages;
     if (smem_for(stages) > 200 * 1024)
       return fail(CT_ERR_UNSUPPORTED, "conv_tc: DCN window does not fit in shared memory%s (%ld)", "", (long)smem_for(stages));
   }
@@ -1326,86 +1212,44 @@ int conv_forward_tc(const ct_conv_desc* d, cudaStream_t st) {
   if (stages > a.k_slices) stages = a.k_slices;
   a.stages = stages;
   const size_t smem = smem_for(stages);
-  {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    static thread_local unsigned long long attr_set_mask = 0;      // the attribute is per device
-    if (dev >= 64 || !((attr_set_mask >> dev) & 1ull)) {
-      CT_CUDA_OK(cudaFuncSetAttribute(conv_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-      CT_CUDA_OK(cudaFuncSetAttribute(conv_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024)));
-      if (dev < 64) attr_set_mask |= 1ull << dev;
-    }
-  }
   const int n_tiles = (g.C_out + n_tile - 1) / n_tile;
-  // Optional 2-D pixel patches (CTB_TC_TILE2D=1) when they tile the map exactly.  Measured on B200: no gain -- the
-  // DCN gather at 128x128 went 150 -> 156 us, level1 184 -> 207 us -- the gather is not L1-capacity bound; off.
-  static const int tile2d_env = getenv("CTB_TC_TILE2D") ? atoi(getenv("CTB_TC_TILE2D")) : 0;
   a.tiles_x = a.tiles_y = 0;
   int m_tiles = (g.P_out + TC_BM - 1) / TC_BM;
-  if (tile2d_env && g.OW % 16 == 0 && g.OH % 8 == 0) {
-    a.tiles_x = g.OW / 16;
-    a.tiles_y = g.OH / 8;
-    m_tiles = g.B * a.tiles_x * a.tiles_y;
-  }
   CUtensorMap tmap;
   memset(&tmap, 0, sizeof(tmap));
   if (win) {                                         // 8x16 patches (ragged at the right / bottom edge) + their windows
     a.tiles_x = (g.OW + 15) / 16;
     a.tiles_y = (g.OH + 7) / 8;
     m_tiles = g.B * a.tiles_x * a.tiles_y;
-    TmapEncodeFn enc = tmap_encode_fn();
-    if (!enc) return fail(CT_ERR_CUDA, "conv_tc: cuTensorMapEncodeTiled entry point unavailable%s", "");
-    const cuuint64_t dims[4] = {(cuuint64_t)g.C_in, (cuuint64_t)g.W, (cuuint64_t)g.H, (cuuint64_t)g.B};
-    const cuuint64_t strides[3] = {(cuuint64_t)g.ld_in * 2, (cuuint64_t)g.W * g.ld_in * 2, (cuuint64_t)g.H * g.W * g.ld_in * 2};
-    const cuuint32_t box[4] = {64, (cuuint32_t)a.win_pw, (cuuint32_t)a.win_ph, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    const CUresult cr = enc(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(d->x), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr != CUDA_SUCCESS) return fail(CT_ERR_CUDA, "conv_tc: cuTensorMapEncodeTiled failed%s (%ld)", "", (long)cr);
-  }
-  static const int persist_env = getenv("CTB_DCN_PERSIST") ? atoi(getenv("CTB_DCN_PERSIST")) : 1;
-  if (win && persist_env && n_tiles == 1 && g.out_mode == CT_OUT_NHWC && d->residual == nullptr && g.C_out % 16 == 0 &&
-      g.C_out == n_tile && ((uintptr_t)d->shift & 15) == 0) {
-    // persistent form: one CTA per SM, two windows + two tables + two accumulators (see dcn_persist_kernel)
+    // persistent form (a single N tile, bf16 NHWC output): one CTA per SM, two windows + two tables + two accumulators,
+    // windows requested one row at a time (see dcn_persist_kernel)
     const size_t win_stride = ((size_t)a.win_bytes + 127) & ~(size_t)127;
     const size_t psmem = (size_t)DP_SA * (A_STAGE_BYTES + n_tile * 128) + 2 * win_stride + 2 * 9 * TC_BM * sizeof(DcnWinEntry) +
                          8 * (2 * DP_SA + 12) + 16 + 1024;
-    if (psmem <= 227 * 1024) {
+    const bool persist = n_tiles == 1 && g.out_mode == CT_OUT_NHWC && d->residual == nullptr && g.C_out % 16 == 0 &&
+                         g.C_out == n_tile && ((uintptr_t)d->shift & 15) == 0 && psmem <= 227 * 1024;
+    const int rc = encode_tmap_nhwc_bf16(&tmap, d->x, g.B, g.H, g.W, g.C_in, g.ld_in, 64, a.win_pw,
+                                         persist ? 1 : a.win_ph, CU_TENSOR_MAP_SWIZZLE_NONE, "conv_tc");
+    if (rc != CT_OK) return rc;
+    if (persist) {
       int cols2 = 32;
       while (cols2 < 2 * n_tile) cols2 <<= 1;
       a.tmem_cols = cols2;
-      int dev = 0, sms = 148;
-      cudaGetDevice(&dev);
-      static thread_local unsigned long long pattr_mask = 0;
-      static thread_local int sms_of[64] = {0};
-      if (dev >= 64 || !((pattr_mask >> dev) & 1ull)) {
-        CT_CUDA_OK(cudaFuncSetAttribute(dcn_persist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024)));
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (dev < 64) { pattr_mask |= 1ull << dev; sms_of[dev] = sms; }
-      } else {
-        sms = sms_of[dev];
-      }
+      CT_CUDA_OK(set_max_dynamic_smem_once((const void*)dcn_persist_kernel, 227 * 1024));
+      const int sms = sm_count();
       const int pgrid = m_tiles < sms ? m_tiles : sms;
-      CUtensorMap tmap_row;                                  // same tensor, one window ROW per request
-      {
-        TmapEncodeFn enc = tmap_encode_fn();
-        const cuuint64_t dims[4] = {(cuuint64_t)g.C_in, (cuuint64_t)g.W, (cuuint64_t)g.H, (cuuint64_t)g.B};
-        const cuuint64_t strides[3] = {(cuuint64_t)g.ld_in * 2, (cuuint64_t)g.W * g.ld_in * 2, (cuuint64_t)g.H * g.W * g.ld_in * 2};
-        const cuuint32_t box[4] = {64, (cuuint32_t)a.win_pw, 1, 1};
-        const cuuint32_t estr[4] = {1, 1, 1, 1};
-        const CUresult cr = enc(&tmap_row, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(d->x), dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (cr != CUDA_SUCCESS) return fail(CT_ERR_CUDA, "conv_tc: cuTensorMapEncodeTiled failed%s (%ld)", "", (long)cr);
-      }
-      CT_CUDA_OK(launch_kernel(dcn_persist_kernel, dim3(pgrid), dim3(DP_THREADS), psmem, st, true, a, m_tiles, tmap_row));
+      CT_CUDA_OK(launch_kernel(dcn_persist_kernel, dim3(pgrid), dim3(DP_THREADS), psmem, st, true, a, m_tiles, tmap));
       return after_launch();
     }
   }
   dim3 grid(m_tiles, n_tiles);
-  if (x3) CT_CUDA_OK(launch_kernel(conv_tc_kernel<true>, grid, dim3(TC_THREADS), smem, st, true, a, tmap));
-  else CT_CUDA_OK(launch_kernel(conv_tc_kernel<false>, grid, dim3(TC_THREADS), smem, st, true, a, tmap));
+  if (x3) {
+    CT_CUDA_OK(set_max_dynamic_smem_once((const void*)conv_tc_kernel<true>, 227 * 1024));
+    CT_CUDA_OK(launch_kernel(conv_tc_kernel<true>, grid, dim3(TC_THREADS), smem, st, true, a, tmap));
+  } else {
+    CT_CUDA_OK(set_max_dynamic_smem_once((const void*)conv_tc_kernel<false>, 200 * 1024));
+    CT_CUDA_OK(launch_kernel(conv_tc_kernel<false>, grid, dim3(TC_THREADS), smem, st, true, a, tmap));
+  }
   return after_launch();
 }
 

@@ -12,7 +12,7 @@
 // memory and selects its top-K there; the last CTA of a batch element to finish merges the C*K candidates by
 // (value, class, index) and writes the K records.
 #include "common.cuh"
-#include <stdlib.h>
+#include "sm100.cuh"
 
 namespace ctb {
 
@@ -21,28 +21,6 @@ constexpr int MAXK = 512;
 constexpr int PEAK_CAP = 4096;   // compact list of kept positive peaks (64-bit keys), 32 KB
 constexpr int PLANE_CAP = 65536; // bytes of one class plane staged in shared memory by bulk copies (128 x 128 fp32)
 constexpr int DEC_NCH = 4;       // ... in this many row chunks, one mbarrier each
-
-// bulk-copy plumbing of the staged plane (the plane of a (b, class) is contiguous in the reference's NCHW layout)
-__device__ __forceinline__ uint32_t dec_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void dec_mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void dec_mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void dec_bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-               "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
-}
-__device__ __forceinline__ void dec_mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  while (!done) {
-    asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    if (++spins > 20000000u) __trap();     // a protocol bug must not hang the GPU
-  }
-}
 
 struct DecodeArgs {
   ct_decode_desc d;
@@ -199,14 +177,14 @@ decode_kernel(DecodeArgs a) {
     if (tid == 0) {
       peak_n = 0; sel_n = 0;
       if (bulk) {
-        for (int c = 0; c < DEC_NCH; ++c) dec_mbar_init(dec_smem_u32(&pbar[c]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (int c = 0; c < DEC_NCH; ++c) mbarrier_init(smem_u32(&pbar[c]), 1);
+        fence_mbarrier_init();
         for (int c = 0; c < DEC_NCH; ++c) {
           const int r0 = c * chunk_rows;
           if (r0 >= H) break;
           const uint32_t bytes = (uint32_t)((H - r0 < chunk_rows ? H - r0 : chunk_rows) * W) * 4u;
-          dec_mbar_expect_tx(dec_smem_u32(&pbar[c]), bytes);
-          dec_bulk_g2s(dec_smem_u32(plane + (size_t)r0 * W), src + (size_t)r0 * W, bytes, dec_smem_u32(&pbar[c]));
+          mbarrier_arrive_expect_tx(smem_u32(&pbar[c]), bytes);
+          cp_async_bulk(smem_u32(plane + (size_t)r0 * W), src + (size_t)r0 * W, bytes, smem_u32(&pbar[c]));
         }
       }
     }
@@ -221,7 +199,7 @@ decode_kernel(DecodeArgs a) {
       if (bulk) {                                       // rows y0-1 .. y0+rpw of this warp: wait for the chunks holding them
         const int y_hi = (y0 + rpw < H ? y0 + rpw : H - 1);
         if (y0 < H)
-          for (int c = 0; c <= y_hi / chunk_rows; ++c) dec_mbar_wait(dec_smem_u32(&pbar[c]), 0u);
+          for (int c = 0; c <= y_hi / chunk_rows; ++c) mbarrier_wait_parity(smem_u32(&pbar[c]), 0u);
       }
       const float* rows = bulk ? plane : src;           // generic pointer: shared or global
       for (int x0 = 0; x0 < W; x0 += 128) {
@@ -532,8 +510,7 @@ extern "C" int ct_decode(const ct_decode_desc* d, void* stream) {
   a.dbg = dec_dbg;
   const int HW = d->H * d->W, K = d->K, J = a.d.J;
   CT_REQUIRE((long long)d->C * HW < (1ll << 31), "C*H*W must stay below 2^31 (class-major positions in the merge keys)");
-  static const int dec_bulk = getenv("CTB_DEC_BULK") ? atoi(getenv("CTB_DEC_BULK")) : 1;
-  a.bulk = (dec_bulk && (size_t)HW * 4 <= PLANE_CAP && (d->W & 3) == 0) ? 1 : 0;      // else: register-streamed planes
+  a.bulk = ((size_t)HW * 4 <= PLANE_CAP && (d->W & 3) == 0) ? 1 : 0;      // else: register-streamed planes
   size_t smem1 = (size_t)PEAK_CAP * 8 + (a.bulk ? PLANE_CAP : 0);
   size_t smem2 = (size_t)(7 * K + 4 * J * K) * 4;
   size_t smem = smem1 > smem2 ? smem1 : smem2;

@@ -1,7 +1,6 @@
 // Bandwidth-bound pieces of the DLA-34 path: the three 7x7 stems (reference NCHW fp32 inputs in,
 // NHWC activations out), Tree.downsample (2x2 max-pool), IDAUp's depthwise transposed-conv
 // upsample fused with the skip add, and the pre_hm gaussian splat.
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace ctb {
@@ -520,8 +519,7 @@ extern "C" int ct_upsample_add(const void* x, const void* skip, const float* w, 
   const size_t total = (size_t)B * H * f * W * f * (C / vec);
   cudaStream_t st = (cudaStream_t)stream;
   const int cv = C / vec;
-  static const int up_mode = getenv("CTB_UP_MODE") ? atoi(getenv("CTB_UP_MODE")) : 1;
-  if (up_mode == 1 && cv <= 256 && 256 % cv == 0 && (256 / cv) % (f * f) == 0 &&
+  if (cv <= 256 && 256 % cv == 0 && (256 / cv) % (f * f) == 0 &&
       (size_t)B * H * f * W * f * (size_t)(ld_out > ld_skip ? ld_out : ld_skip) < (1ull << 31) && (size_t)B * H * W * ld_in < (1ull << 31)) {
     // all phases of an input pixel in one CTA (L1 reuse of the taps); grid: a few CTAs per SM, grid-stride over pixels
     const int per_cta = (256 / cv) / (f * f);

@@ -21,6 +21,7 @@ precision='bf16x3' : fp32 activations, tcgen05 gather engine with bf16 hi/lo spl
 precision='fp32'   : fp32 activations, SIMT engine (reference-accuracy path, <= 1e-3 of the reference)
 """
 import ctypes as C
+import os
 
 import numpy as np
 import torch
@@ -43,13 +44,6 @@ class TV(object):
 
   def tensor(self):
     return self.buf[..., self.off:self.off + self.C]
-
-
-def _pow2_at_least(n):
-  p = 16
-  while p < n:
-    p *= 2
-  return p
 
 
 def s2d_weights_3x3_s1(w):
@@ -88,7 +82,7 @@ def s2d_weights_3x3_s2(w):
 class DLA34Engine(object):
 
   def __init__(self, state_dict, heads, B, H, W, precision='bf16', device='cuda',
-               depth_scale=1.0, has_pre_img=True, has_pre_hm=True, use_halo=True, dla_node='dcn'):
+               depth_scale=1.0, has_pre_img=True, has_pre_hm=True, dla_node='dcn'):
     assert precision in ('bf16', 'fp32', 'bf16x3')
     assert dla_node in ('dcn', 'conv', 'gcn')
     self.dla_node = dla_node
@@ -104,11 +98,6 @@ class DLA34Engine(object):
     self.ct_dtype = L.CT_BF16 if precision == 'bf16' else L.CT_F32
     self.engine = {'bf16': L.CT_ENGINE_TCGEN05, 'fp32': L.CT_ENGINE_SIMT, 'bf16x3': L.CT_ENGINE_TCGEN05_X3}[precision]
     self.x3 = (precision == "bf16x3")
-    self.dcn_window = bool(int(__import__('os').environ.get('CTB_DCN_WINDOW', '1')))
-    # the persistent window kernel (CTB_DCN_PERSIST, default on) also wins on 128 -> 128 at 64x64 (100 vs 124 us)
-    self.dcn_window_all = bool(int(__import__('os').environ.get('CTB_DCN_PERSIST', '1')))
-    self.ntile_cap = int(__import__('os').environ.get('CTB_NTILE_CAP', '256'))
-    self.gather_128 = bool(int(__import__('os').environ.get('CTB_GATHER_128', '0')))   # experiment: level3's 3x3 on the gather engine
     self.depth_scale = float(depth_scale)
     self.has_pre_img = has_pre_img and ('base.pre_img_layer.0.weight' in self.sd)
     self.has_pre_hm = has_pre_hm and ('base.pre_hm_layer.0.weight' in self.sd)
@@ -119,10 +108,8 @@ class DLA34Engine(object):
     self.algo_flops = {}   # op name -> flops of the reference layer, where the launch shape carries structural zeros
     self.s2d_named = set() # named intermediates stored space-to-depth ([B, H/2, W/2, (sy, sx, 16)])
     self.n_sm = 148
-    self.debug_sync = bool(int(__import__('os').environ.get('CTB_DEBUG_SYNC', '0')))
-    self.use_halo = use_halo and precision == 'bf16'
-    # level1 as a 2x2 stride-1 halo convolution over level0's output written space-to-depth (see _build)
-    self.s2d_level1 = bool(int(__import__('os').environ.get('CTB_S2D_LEVEL1', '1'))) and self.use_halo
+    self.debug_sync = bool(int(os.environ.get('CTB_DEBUG_SYNC', '0')))
+    self.use_halo = precision == 'bf16'
     self._build()
     self.graph = None
 
@@ -189,15 +176,10 @@ class DLA34Engine(object):
     P = self.B * OH * OW
     engine = self.engine
     n_tile = self._pick_n_tile(P, C_out) if engine in (L.CT_ENGINE_TCGEN05, L.CT_ENGINE_TCGEN05_X3) else 0
-    if engine == L.CT_ENGINE_TCGEN05 and a_mode == L.CT_A_CONV and n_tile > self.ntile_cap:
-      # experiment knob (CTB_NTILE_CAP): 128-wide tiles with two co-resident CTAs measured SLOWER than one 256-wide
-      # CTA on levels 4-5 (conv_tc plain 1.81 vs 1.73 ms per 32-frame step), so the default cap is 256 = no cap
-      n_tile = self.ntile_cap
     if engine == L.CT_ENGINE_TCGEN05_X3 and n_tile > 128 and a_mode == L.CT_A_DCN:
       n_tile = 128            # x3 DCN: two 36 KB-table stages of (32 + 2 x n_tile/8) KB must fit
     if engine == L.CT_ENGINE_TCGEN05 and self.use_halo and a_mode == L.CT_A_CONV and stride == 1 and kh == kw and \
-        (C_in in (16, 32, 48, 64, 128, 192, 256) or (C_in == 8 and sum3)) and \
-        not (self.gather_128 and C_in == 128 and C_out == 128 and kh == 3):
+        (C_in in (16, 32, 48, 64, 128, 192, 256) or (C_in == 8 and sum3)):
       k = kh
       # stride-1 layer whose weights fit in smem: TMA halo tile + descriptor-shifted taps (csrc/conv_halo.cu)
       nblk = k * ((k + 1) // 2) if C_in == 8 else k * k * (C_in // 16)
@@ -274,11 +256,9 @@ class DLA34Engine(object):
                sd[p + '.conv.conv_offset_mask.bias'], om, 3, 1, relu=False,
                out_mode=L.CT_OUT_NHWC_F32, sig_from=18)
     w, shift = self._fold(p + '.conv', p + '.actf.0')
-    # window sampler; without the persistent kernel its smem footprint (18 KB table + 43 KB window + stages) halves the
-    # occupancy of a layer whose N tile is wide and whose input needs two window refills (128 -> 128 at 64x64: 155 vs 136 us)
-    if (self.engine == L.CT_ENGINE_TCGEN05 and x.C % 64 == 0 and self.dcn_window and
-        (self.dcn_window_all or not (x.C == 128 and w.shape[0] == 128))):
-      # sample from a TMA-staged shared-memory window; K order = (64-channel chunk, tap, channel)
+    if self.engine == L.CT_ENGINE_TCGEN05 and x.C % 64 == 0:
+      # sample from a TMA-staged shared-memory window; K order = (64-channel chunk, tap, channel).  With the persistent
+      # window kernel this also wins on 128 -> 128 at 64x64 (100 vs 124 us for the global-memory sampler)
       nch = x.C // 64
       w_cm = w.reshape(w.shape[0], nch, 64, 3, 3).permute(0, 2, 1, 3, 4).reshape(w.shape[0], 64, nch * 3, 3)
       self._conv(p, x, w, shift, out, 3, 1, relu=True, a_mode=L.CT_A_DCN_WIN, om=om, w_pack=w_cm.contiguous())
@@ -348,7 +328,7 @@ class DLA34Engine(object):
       shst[si] = sh
     self.stem_w = self._dev(wst.to(f32).contiguous())
     self.stem_shift = self._dev(shst.to(f32).contiguous())
-    s2d = self.s2d_level1 and H % 2 == 0 and W % 2 == 0      # stem -> level0 -> level1 on the space-to-depth grid
+    s2d = self.use_halo and H % 2 == 0 and W % 2 == 0      # stem -> level0 -> level1 on the space-to-depth grid
     x0 = TV(self._buf(H // 2, W // 2, 64), 0, 64) if s2d else TV(self._buf(H, W, 16), 0, 16)
     if self.use_halo:
       # tensor-core stem: pack (img, pre, hm) -> bf16 NHWC [.,8], one 7x7 conv 8 -> 48 (block-diagonal over the

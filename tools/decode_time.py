@@ -45,5 +45,5 @@ for kind in ('iid', 'smooth'):
     torch.cuda.synchronize()
     ts.append(e0.elapsed_time(e1) * 1000)
   ts.sort()
-  print('%s maps, CTB_DEC_DEBUG=%s CTB_DEC_BULK=%s: median %.1f us, min %.1f us' % (
-      kind, os.environ.get('CTB_DEC_DEBUG', '0'), os.environ.get('CTB_DEC_BULK', '1'), ts[len(ts) // 2], ts[0]))
+  print('%s maps, CTB_DEC_DEBUG=%s: median %.1f us, min %.1f us' % (
+      kind, os.environ.get('CTB_DEC_DEBUG', '0'), ts[len(ts) // 2], ts[0]))

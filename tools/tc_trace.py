@@ -57,7 +57,7 @@ for (name, B, Cin, Cout, H, W, k, stride, dcn, nt) in cases:
   torch.cuda.synchronize()
   L.check(lib.ct_debug_trace(None))
   t = tr.cpu().numpy().astype(np.int64)
-  if os.environ.get('CTB_DCN_PERSIST', '1') == '1' and dcn == 'win':      # the persistent window kernel (default on)
+  if dcn == 'win':                                       # the persistent window kernel
     q = t[16:16 + 240].reshape(60, 4)
     n = int((q[:, 3] > 0).sum())
     base = q[0, 0]
